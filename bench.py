@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- rule-grounded queries/sec on the FB15k-237-shaped synthetic workload.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step = one pass of the hot path (ground every rule of the head -> candidate cells -> rule-weight aggregation ->
@@ -281,6 +281,7 @@ class Runner:
         torch.cuda.synchronize()
         if self.world > 1:
             torch.distributed.barrier()
+        self.last_step = (loss, tsum, gbuf)
         ms = ev0.elapsed_time(ev1)
         if dbg and len(step_ev) > 1:
             per = [step_ev[i].elapsed_time(step_ev[i + 1]) for i in range(len(step_ev) - 1)]
@@ -446,6 +447,18 @@ def dense_expansion_traffic(kg, cr, heads):
     return float(head_bytes[heads].sum())
 
 
+def dump_outputs(out_dir, model, loss, tsum, gbuf):
+    """What the last timed step hands its caller, as float32 DIR/<name>.npy: the loss and target sum of each batch, the
+    gradients it accumulated and the parameters after its optimizer step (1.2 MB on the fb15k237 shape)."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss, "target_sum": tsum, "rule_weights_grad": gbuf.view(model.rule_weights),
+              "bias_grad": gbuf.view(model.bias), "rule_weights": model.rule_weights, "bias": model.bias}
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def reduce_max_sum(ms, q, dev, world):
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     n = torch.tensor([q], dtype=torch.float64, device=dev)
@@ -562,7 +575,11 @@ def main():
     ap.add_argument("--typed", action="store_true", help="headline on the typed synthetic graph instead of the i.i.d. one")
     ap.add_argument("--shape", default="fb15k237", choices=["fb15k237", "wn18rr"],
                     help="synthetic workload shape (the headline metric is quoted on fb15k237)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed headline step computed to DIR/<name>.npy "
+                    "(inputs are seeded: two builds compare output for output)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
 
@@ -628,6 +645,8 @@ def main():
         clocks.start()
     # ---------------- device-resident timing (`value`) ----------------
     elapsed_ms, q_timed, launches, level_events = run.device_loop(args.warmup, args.steps, level_events=True)
+    if args.dump_outputs and rank == 0:          # before the end-to-end loop trains the model further
+        dump_outputs(args.dump_outputs, model, *run.last_step)
     step_ms_local = elapsed_ms
     elapsed_ms, q_total = reduce_max_sum(elapsed_ms, q_timed, dev, world)
     value = q_total / (elapsed_ms / 1e3)

@@ -178,50 +178,42 @@ def test_world2_gloo_collectives(tmp_path):
     assert len(r0["mine"]) == len(r1["mine"]) == 5 and set(r0["mine"]) | set(r1["mine"]) == set(range(9))
 
 
-def test_compat_modules_resolve_the_reference_scripts_imports(monkeypatch):
+def test_compat_modules_resolve_the_reference_scripts_imports(monkeypatch, tmp_path):
     """`from data import ...`, `from predictors import ...`, ... of run_predictorplus.py / run_rnnlogic.py
     resolve through compat/ (names only; running them needs a GPU).  Generator-side names come from the
-    reference's own files when its src/ is on the path."""
-    import ast
+    reference's own files when its src/ follows compat/ on the path: a stand-in src/ that defines only
+    those names takes its place here."""
     import importlib
     import sys
-    import types
     compat = os.path.join(G.ROOT, "compat")
-    ref_src = "/root/reference/src"
     monkeypatch.syspath_prepend(compat)
-    for m in ("data", "predictors", "trainer", "comm", "utils", "_reference"):
+    for m in ("data", "predictors", "trainer", "comm", "utils", "_reference", "generators"):
         sys.modules.pop(m, None)
     wanted = {"data": ["KnowledgeGraph", "TrainDataset", "ValidDataset", "TestDataset"],
               "predictors": ["Predictor", "PredictorPlus"], "trainer": ["TrainerPredictor"],
               "utils": ["load_config", "save_config", "set_logger", "set_seed"], "comm": ["get_rank"]}
-    if os.path.isdir(ref_src):                                   # read the real import lists
-        for script in ("run_predictorplus.py", "run_rnnlogic.py"):
-            tree = ast.parse(open(os.path.join(ref_src, script)).read())
-            for node in ast.walk(tree):
-                if isinstance(node, ast.ImportFrom) and node.module in wanted:
-                    wanted[node.module] += [a.name for a in node.names]
-    generator_side = {"RuleDataset", "Iterator", "TrainerGenerator"}
     for mod, names in wanted.items():
         module = importlib.import_module(mod)
         assert os.path.dirname(module.__file__) == compat
-        for n in set(names) - generator_side:
+        for n in names:
             assert hasattr(module, n), (mod, n)
-    if os.path.isdir(ref_src):
-        # generator-side classes are fetched from the reference's files (needs its third-party imports)
-        ts = types.ModuleType("torch_scatter")
-        ts.scatter = ts.scatter_add = ts.scatter_min = ts.scatter_max = ts.scatter_mean = None
-        ed = types.ModuleType("easydict")
-        ed.EasyDict = dict
-        monkeypatch.setitem(sys.modules, "torch_scatter", ts)
-        monkeypatch.setitem(sys.modules, "easydict", ed)
-        sys.path.append(ref_src)
-        try:
-            import trainer
-            import data
-            assert trainer.TrainerGenerator.__module__ == "_reference_trainer"
-            assert data.RuleDataset.__module__ == "_reference_data"
-        finally:
-            sys.path.remove(ref_src)
+    import data
+    with pytest.raises(AttributeError, match="outside the B200 hot path"):
+        data.RuleDataset
+    ref_src = tmp_path / "src"
+    ref_src.mkdir()
+    generator_side = {"data": ["RuleDataset", "Iterator"], "trainer": ["TrainerGenerator"], "generators": ["Generator"]}
+    for mod, names in generator_side.items():
+        (ref_src / (mod + ".py")).write_text("".join("class %s:\n    pass\n" % n for n in names))
+    sys.path.append(str(ref_src))
+    try:
+        for mod, names in generator_side.items():
+            module = importlib.import_module(mod)
+            assert os.path.dirname(module.__file__) == compat
+            for n in names:
+                assert getattr(module, n).__module__ == "_reference_" + mod, (mod, n)
+    finally:
+        sys.path.remove(str(ref_src))
     for m in ("data", "predictors", "trainer", "comm", "utils", "_reference", "generators"):
         sys.modules.pop(m, None)
 
