@@ -29,7 +29,7 @@ extern "C" {
 #endif
 
 #define RL_LANES 32
-#define RL_ABI_VERSION 4
+#define RL_ABI_VERSION 5
 
 enum rl_status {
     RL_OK = 0,
@@ -258,14 +258,7 @@ int rl_softmax_ce(const rl_graph *g, const rl_slots *s, const rl_answers *train_
                   int32_t n_groups, const int32_t *group_ptr, float *partial, float *stats,
                   float *slot_sums, float *group_loss, float *group_tsum, float *G, void *stream);
 
-/* Kernel (2c): backward into rule weights and bias, replaces autograd through
- * src/predictors.py:64,74.  grad_w[num_rules] and grad_bias[N] (may be NULL) are ACCUMULATED
- * into (zero them first): grad_w[i] += sum_s slot_scale[s] * <G_s, fp32(count_i)>. */
-int rl_predictor_backward(const rl_graph *g, const rl_rules *r, const rl_slots *s,
-                          const rl_frontier *fr, const float *G, const float *slot_scale,
-                          float *grad_w, float *grad_bias, void *stream);
-
-/* Kernels (2b)+(2c) in one call for Predictor's train step (src/trainer.py:84,88-90 + autograd
+/* Kernel (2b) fused with the backward into rule weights and bias for Predictor's dense train step (src/trainer.py:84,88-90 + autograd
  * through src/predictors.py:64,74): same loss outputs and scratch as rl_softmax_ce, then the
  * backward with the passes fused (softmax gradient + bias gradient in one sweep over Z, target
  * terms pushed into G and grad_bias together, item walk over the entity-grouped list).
@@ -365,24 +358,6 @@ int rl_lstm_encode_backward(int32_t n, int32_t T, int32_t H, int32_t L, const in
 int rl_lstm_encode_wgrad(int64_t M, int32_t H, int32_t L, const float *dG, const float *ih, float *dW,
                          float *db, void *stream);
 
-/* Fused dense tail of PredictorPlus with the `sum` aggregator, one thread per candidate cell
- * (src/layers.py:73-75: Linear(H,H) -> LayerNorm -> ReLU; src/predictors.py:253-255: concat with
- * relation_emb[head], Linear(2H,J) -> ReLU -> Linear(J,1)).  F[C][H] from rl_plus_features,
- * cand_head[C] the head relation of each candidate's query, z[C] the candidate scores.  H in {16,32},
- * J <= 256; row-major weights as in torch (W0[H][H], W1[J][2H], W2[J]). */
-int rl_sum_tail_forward(int64_t C, int32_t H, int32_t J, const float *F, const int32_t *cand_head,
-                        const float *W0, const float *b0, const float *gamma, const float *beta,
-                        const float *W1, const float *b1, const float *W2, const float *b2,
-                        const float *rel_emb, float *z, void *stream);
-/* Backward: recomputes the forward; writes dF[C][H] and the per-candidate factors delta1[C][J],
- * U[C][2H], dY[C][H], dRel[C][H] (dW1 = delta1^T U, dW0 = dY^T F, d relation_emb = index_add(dRel));
- * ACCUMULATES the small gradients into g_small = [b0 H | gamma H | beta H | b1 J | W2 J | b2 1]. */
-int rl_sum_tail_backward(int64_t C, int32_t H, int32_t J, const float *F, const int32_t *cand_head,
-                         const float *W0, const float *b0, const float *gamma, const float *beta,
-                         const float *W1, const float *b1, const float *W2, const float *b2,
-                         const float *rel_emb, const float *dz, float *dF, float *delta1, float *U,
-                         float *dY, float *dRel, float *g_small, void *stream);
-
 /* ---- RotatE entity feature (src/embedding.py:28-70) -----------------------------------------
  * out[S][N][32] = gamma - sum_d |h_b o rot(remb[head]) - e|_d for every entity e; eemb fp32[N][2D]
  * (re | im), remb fp32[R][D] (already doubled with the negated copy, embedding.py:23-26).
@@ -409,9 +384,10 @@ int rl_mask_to_dense(int32_t N, int32_t nq, const uint32_t *nzmask_slot, uint8_t
 
 /* ---- the scoring half on candidate cells (rl_cells.cu, rl_tail_tc.cu): no [S][N][32] matrix ---- */
 
-/* Number the cells: cand_off, cell_key, cell_ent, slot_ncell, counters[0..1] from the candidate words nzmask.  When
- * the frontier carries sort buffers the items are grouped by entity first (rl_sort_items, which ORs their lane
- * masks into nzmask).  Replaces torch.nonzero(mask) (src/predictors.py:239) without a host sync. */
+/* Number the cells: cand_off, cell_key, cell_ent, slot_ncell, counters[0..1] from the candidate words nzmask that
+ * k_numeric left (the frontier must be expanded without sort buffers, bucket_cnt == NULL; RL_ERR_ARG otherwise);
+ * the cells of empty-body rules are added to nzmask here.  counters[0] counts every cell, also those beyond cap.
+ * Replaces torch.nonzero(mask) (src/predictors.py:239) without a host sync. */
 int rl_cells_build(const rl_graph *g, const rl_rules *r, const rl_slots *s, const rl_frontier *fr,
                    const rl_cells *c, void *stream);
 
@@ -419,15 +395,12 @@ int rl_cells_build(const rl_graph *g, const rl_rules *r, const rl_slots *s, cons
  * rl_cells_softmax_ce.  Once per parameter update. */
 int rl_bias_stats(int32_t N, const float *bias, double *acc, void *stream);
 
-/* Predictor (src/predictors.py:58-65): zc[cell] = sum_rule w_rule * fp32(count), without the bias.
- * _item_: one THREAD per item (non-zero row of a rule-end node) in the order k_numeric appended them: it reads the
- *         counts of the queries in the item's lane mask and adds w * fp32(count) to their cells (zc[cap] is cleared
- *         first); no sort, no per-warp walk of ragged lists;
- * _cell_: one warp per 32 entities over the entity-grouped items (frontier with sort buffers; deterministic sums). */
+/* Predictor (src/predictors.py:58-65): zc[cell] = sum_rule w_rule * fp32(count), without the bias.  One THREAD per
+ * item (non-zero row of a rule-end node) in the order k_numeric appended them: it reads the counts of the queries in
+ * the item's lane mask and adds w * fp32(count) to their cells (zc[cap] is cleared first); no sort, no per-warp walk
+ * of ragged lists. */
 int rl_predictor_item_scores(const rl_graph *g, const rl_rules *r, const rl_slots *s, const rl_frontier *fr,
                             const rl_cells *c, const float *w, float *zc, void *stream);
-int rl_predictor_cell_scores(const rl_graph *g, const rl_rules *r, const rl_slots *s, const rl_frontier *fr,
-                             const rl_cells *c, const float *w, float *zc, void *stream);
 
 /* log(softmax + 1e-8) cross-entropy against the smoothed multi-hot target (src/trainer.py:84,88-89) with the
  * logits given as cell scores zc plus bias[e] for EVERY entity (bias != NULL; predictors.py:257-262), or as
@@ -444,8 +417,6 @@ int rl_cells_softmax_ce(const rl_graph *g, const rl_slots *s, const rl_cells *c,
  * item and rule). */
 int rl_predictor_item_backward(const rl_graph *g, const rl_rules *r, const rl_slots *s, const rl_frontier *fr,
                               const rl_cells *c, const float *Gc, float *grad_w, void *stream);
-int rl_predictor_cell_backward(const rl_graph *g, const rl_rules *r, const rl_slots *s, const rl_frontier *fr,
-                               const rl_cells *c, const float *Gc, float *grad_w, void *stream);
 
 /* Filtered rank (src/trainer.py:189-201) from cell scores: (L,H) int64[S*32][2].  With a bias the entities
  * outside a query's cells are counted by binary search in sorted_bias (bias sorted ascending);
@@ -454,25 +425,20 @@ int rl_cells_rank(const rl_graph *g, const rl_slots *s, const rl_cells *c, const
                   const float *bias, const float *sorted_bias, const float *zc, int32_t *counters, int64_t *LH,
                   void *stream);
 
-/* Z[S][N][32] += zc at the cells / Gc = G at the cells (dense entity features such as RotatE, API forward). */
+/* Z[S][N][32] += zc at the cells / Gc = G at the cells (dense entity features such as RotatE; the [B,N] scores of
+ * the reference's forward()). */
 int rl_cells_add_to_dense(const rl_graph *g, const rl_slots *s, const rl_cells *c, const float *zc, float *Z, void *stream);
 int rl_cells_gather_dense(const rl_graph *g, const rl_slots *s, const rl_cells *c, const float *G, float *Gc, void *stream);
 
-/* PredictorPlus aggregates per cell (src/layers.py:68-72 / 92-99), hidden_dim 16, emb[num_rules][16] indexed by
- * the global rule id.  _item_: F[cell][16] = sum fp32(count) * emb[rule], one thread per (item, quarter of the
- * hidden vector), 16-byte vector atomics (F[cap][16] is cleared first).  _cell_: from the entity-grouped items (also the PNA statistics
- * out_sq, out_min, out_max, arg_min, arg_max, degree[cell]). */
+/* PredictorPlus sum aggregate per cell (src/layers.py:68-72), hidden_dim 16, emb[num_rules][16] indexed by the global
+ * rule id: F[cell][16] = sum fp32(count) * emb[rule], one thread per (item, quarter of the hidden vector), 16-byte
+ * vector atomics (F[cap][16] is cleared first).  The PNA statistics come from rl_pna_item_stats. */
 int rl_plus_item_features(const rl_graph *g, const rl_rules *r, const rl_slots *s, const rl_frontier *fr,
                          const rl_cells *c, const float *emb, int32_t H, float *F, void *stream);
-int rl_plus_cell_features(const rl_graph *g, const rl_rules *r, const rl_slots *s, const rl_frontier *fr,
-                          const rl_cells *c, const float *emb, int32_t H, int32_t pna, float *out_sum, float *out_sq,
-                          float *out_min, float *out_max, int32_t *arg_min, int32_t *arg_max, float *degree, void *stream);
 
 /* grad_emb[rule][16] += sum over the rule's non-zero counts of fp32(count) * dF[cell][16]. */
 int rl_plus_item_backward(const rl_graph *g, const rl_rules *r, const rl_slots *s, const rl_frontier *fr,
                          const rl_cells *c, int32_t H, const float *dF, float *grad_emb, void *stream);
-int rl_plus_cell_backward(const rl_graph *g, const rl_rules *r, const rl_slots *s, const rl_frontier *fr,
-                          const rl_cells *c, int32_t H, const float *dF, float *grad_emb, void *stream);
 
 /* Dense tail of PredictorPlus on the cells (src/layers.py:73-75, src/predictors.py:253-255), H = 16, J = 128:
  * zc[cell] = W2 . relu(W1 [relu(LN(W0 F + b0)), rel[head]] + b1) + b2  (rl_tail_tc.cu).  The Linear(2H,128) of the

@@ -12,7 +12,7 @@ import subprocess
 _HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(_HERE)
 LIB_PATH = os.environ.get("RNNLOGIC_B200_LIB") or os.path.join(_HERE, "lib", "librnnlogic_b200.so")   # env override: A/B builds
-SOURCES = [os.path.join(_HERE, "csrc", f) for f in ("rl_kernels.cu", "rl_cells.cu", "rl_plus.cu", "rl_rotate.cu", "rl_tail.cu", "rl_tail_tc.cu", "rl_pna.cu", "rl_rnn.cu", "rl_miner.cu")]
+SOURCES = [os.path.join(_HERE, "csrc", f) for f in ("rl_kernels.cu", "rl_cells.cu", "rl_plus.cu", "rl_rotate.cu", "rl_tail_tc.cu", "rl_pna.cu", "rl_rnn.cu", "rl_miner.cu")]
 HEADER = os.path.join(ROOT, "include", "rnnlogic_b200.h")
 
 LANES = 32
@@ -137,8 +137,6 @@ _PROTOS = {
     "rl_softmax_blocks": (C.c_int, [C.c_int32]),
     "rl_softmax_ce": (C.c_int, [C.POINTER(RlGraph), C.POINTER(RlSlots), C.POINTER(RlAnswers), C.c_float,
                                 C.c_int32, vp, vp, C.c_int32, vp, vp, vp, vp, vp, vp, vp, vp]),
-    "rl_predictor_backward": (C.c_int, [C.POINTER(RlGraph), C.POINTER(RlRules), C.POINTER(RlSlots),
-                                        C.POINTER(RlFrontier), vp, vp, vp, vp, vp]),
     "rl_filtered_rank": (C.c_int, [C.POINTER(RlGraph), C.POINTER(RlSlots), C.POINTER(RlAnswers), C.c_int32,
                                    vp, vp, vp, vp, vp]),
     "rl_filtered_rank_dense": (C.c_int, [C.c_int64, C.c_int64, vp, vp, vp, vp, vp, vp]),
@@ -152,16 +150,12 @@ _PROTOS = {
     "rl_plus_gather": (C.c_int, [C.POINTER(RlGraph), C.POINTER(RlSlots), vp, vp, vp, vp, vp]),
     "rl_plus_backward": (C.c_int, [C.POINTER(RlGraph), C.POINTER(RlRules), C.POINTER(RlSlots), C.POINTER(RlFrontier),
                                    vp, vp, vp, C.c_int32, vp, vp, C.c_int32, vp, vp, vp]),
-    "rl_sum_tail_forward": (C.c_int, [C.c_int64, C.c_int32, C.c_int32] + [vp] * 13),
-    "rl_sum_tail_backward": (C.c_int, [C.c_int64, C.c_int32, C.c_int32] + [vp] * 19),
     "rl_rotate_scores": (C.c_int, [C.POINTER(RlGraph), C.POINTER(RlSlots), C.c_int32, C.c_float, vp, vp, vp, vp, vp]),
     "rl_rotate_backward": (C.c_int, [C.POINTER(RlGraph), C.POINTER(RlSlots), C.c_int32, C.c_float, vp, vp, vp, vp, vp,
                                      vp, vp, vp]),
     "rl_cells_build": (C.c_int, [C.POINTER(RlGraph), C.POINTER(RlRules), C.POINTER(RlSlots), C.POINTER(RlFrontier),
                                  C.POINTER(RlCells), vp]),
     "rl_bias_stats": (C.c_int, [C.c_int32, vp, vp, vp]),
-    "rl_predictor_cell_scores": (C.c_int, [C.POINTER(RlGraph), C.POINTER(RlRules), C.POINTER(RlSlots),
-                                           C.POINTER(RlFrontier), C.POINTER(RlCells), vp, vp, vp]),
     "rl_predictor_item_scores": (C.c_int, [C.POINTER(RlGraph), C.POINTER(RlRules), C.POINTER(RlSlots),
                                           C.POINTER(RlFrontier), C.POINTER(RlCells), vp, vp, vp]),
     "rl_cells_softmax_ce": (C.c_int, [C.POINTER(RlGraph), C.POINTER(RlSlots), C.POINTER(RlCells), C.POINTER(RlAnswers),
@@ -170,18 +164,12 @@ _PROTOS = {
                                        C.POINTER(RlCells), vp, C.c_int32, vp, vp]),
     "rl_plus_item_backward": (C.c_int, [C.POINTER(RlGraph), C.POINTER(RlRules), C.POINTER(RlSlots), C.POINTER(RlFrontier),
                                        C.POINTER(RlCells), C.c_int32, vp, vp, vp]),
-    "rl_predictor_cell_backward": (C.c_int, [C.POINTER(RlGraph), C.POINTER(RlRules), C.POINTER(RlSlots),
-                                             C.POINTER(RlFrontier), C.POINTER(RlCells), vp, vp, vp]),
     "rl_predictor_item_backward": (C.c_int, [C.POINTER(RlGraph), C.POINTER(RlRules), C.POINTER(RlSlots),
                                             C.POINTER(RlFrontier), C.POINTER(RlCells), vp, vp, vp]),
     "rl_cells_rank": (C.c_int, [C.POINTER(RlGraph), C.POINTER(RlSlots), C.POINTER(RlCells), C.POINTER(RlAnswers),
                                 vp, vp, vp, vp, vp, vp]),
     "rl_cells_add_to_dense": (C.c_int, [C.POINTER(RlGraph), C.POINTER(RlSlots), C.POINTER(RlCells), vp, vp, vp]),
     "rl_cells_gather_dense": (C.c_int, [C.POINTER(RlGraph), C.POINTER(RlSlots), C.POINTER(RlCells), vp, vp, vp]),
-    "rl_plus_cell_features": (C.c_int, [C.POINTER(RlGraph), C.POINTER(RlRules), C.POINTER(RlSlots), C.POINTER(RlFrontier),
-                                        C.POINTER(RlCells), vp, C.c_int32, C.c_int32, vp, vp, vp, vp, vp, vp, vp, vp]),
-    "rl_plus_cell_backward": (C.c_int, [C.POINTER(RlGraph), C.POINTER(RlRules), C.POINTER(RlSlots), C.POINTER(RlFrontier),
-                                        C.POINTER(RlCells), C.c_int32, vp, vp, vp]),
     "rl_pair_table": (C.c_int, [C.POINTER(RlGraph), C.c_int32, vp, vp, vp, vp, vp, vp]),
     "rl_mine_rules": (C.c_int, [C.c_int32, vp, vp, vp, vp, C.c_int32, C.c_int32, vp, C.c_int64, vp, vp]),
     "rl_tail_scratch_floats": (C.c_int64, [C.c_int32]),

@@ -189,10 +189,9 @@ PLUS_PLANES = 2 + 4 * 16 + 4          # zc, Gc | F, dF, O, dY [16 each] | ReLU b
 PNA_PLANES = PLUS_PLANES + 16 + 16 + 32 + 32 + 64 + 64 + 2    # + s1, s2 | min keys, max keys (u64 x 16) | FEAT | dstat | deg, SC
 
 
-def _plus_planes(gr, pna=False):
-    """Per-cell arrays of the PredictorPlus step inside the grounder's cell workspace (contiguous [cap][16] blocks)."""
-    cap, ws = gr._ws_cells_cap, gr._ws_cells
-    blk = lambda i0, n: ws[(2 + i0) * cap:(2 + i0 + n) * cap]          # plane 0: cell keys, plane 1: cell entities
+def _plus_planes(planes, pna=False):
+    """Per-cell arrays of the PredictorPlus step in the planes of build_cells (contiguous [cap][16] blocks)."""
+    blk = lambda i0, n: planes[i0:i0 + n].view(-1)
     pl = {"zc": blk(0, 1), "Gc": blk(1, 1), "F": blk(2, 16), "dF": blk(18, 16), "O": blk(34, 16), "dY": blk(50, 16),
           "bits": blk(66, 4)}
     if pna:
@@ -223,20 +222,52 @@ def _step_rule_ids(model, sl, device):
     return torch.from_numpy(ids).to(device, non_blocking=True)
 
 
+def _encode_rules(model, ids):
+    """Output of the rule encoder (rnn / lstm / gru) for the rules ``ids``, with autograd when it is enabled."""
+    if model.rule_features.device != ids.device:
+        model.rule_features = model.rule_features.to(ids.device)
+    return model.encode_rules(model.rule_features[ids])
+
+
 def _rule_embeddings(model, sl, device):
-    """-> (emb [num_rules,16] fp32 indexed by global rule id, backward closure(grad_emb) or None)."""
+    """-> (emb [num_rules,16] fp32 indexed by global rule id, (ids, encoder output) or None)."""
     if model.type == "emb":
         return model.rule_emb.detach(), None
     ids = _step_rule_ids(model, sl, device)
-    if model.rule_features.device != device:
-        model.rule_features = model.rule_features.to(device)
     full = model._emb_scratch(device)
     if ids.numel() == 0:
         return full, None
     with torch.enable_grad():
-        sub = model.encode_rules(model.rule_features[ids])                    # rule encoder: small autograd graph
+        sub = _encode_rules(model, ids)                                       # rule encoder: small autograd graph
     full.index_copy_(0, ids, sub.detach().float())
     return full, (ids, sub)
+
+
+def _plus_scores(model, ck, sl, pl, emb, wts):
+    """Forward half of a PredictorPlus step on the cells: aggregate the rule embeddings ``emb`` (sum, or the PNA
+    statistics + front) -> dense tail -> pl["zc"]."""
+    pna = model.aggregator == "pna"
+    if pna:                                                              # statistics -> scalers + Linear(12H,H) -> F holds y
+        ck.pna_stats(sl, emb, pl["pna"])
+        ck.pna_front_forward(sl, pl["pna"], wts[0], wts[1], pl["F"], pl["FEAT"], pl["SC"])
+    else:
+        ck.plus_features(sl, emb, pl["F"])
+    ck.tail_forward(sl, pl["F"], wts, pl["zc"], pl["bits"], front_done=pna)
+
+
+def _plus_backward(model, ck, sl, pl, emb, wts, grads, grad_emb):
+    """Backward half: pl["Gc"] -> dense tail -> aggregate.  ACCUMULATES into ``grads`` (the _tail_weights) and
+    ``grad_emb`` [num_rules,16] (None: the step has no rule to take a gradient)."""
+    pna = model.aggregator == "pna"
+    ck.tail_backward(sl, model.num_relations, pl["F"], wts, pl["Gc"], pl["bits"], pl["dF"], pl["dY"], grads,
+                     model._d1sum_scratch(ck.device), front_done=pna)
+    if grad_emb is None:
+        return
+    if pna:
+        ck.pna_front_backward(sl, pl["pna"], wts[0], pl["dY"], pl["FEAT"], pl["SC"], pl["dstat"], grads[0])
+        ck.pna_backward(sl, emb, pl["pna"], pl["dstat"], grad_emb)
+    else:
+        ck.plus_backward(sl, pl["dF"], grad_emb)
 
 
 def plus_step(model, sk, sl, smoothing, grad_scale, gbuf: GradBuffer, expanded=False, bits=32, want_grad=True):
@@ -248,17 +279,12 @@ def plus_step(model, sk, sl, smoothing, grad_scale, gbuf: GradBuffer, expanded=F
     if not expanded:
         sk.gr._run(sl, bits)
     pna = model.aggregator == "pna"
-    sk.gr.build_cells(sl, PNA_PLANES if pna else PLUS_PLANES)
-    pl = _plus_planes(sk.gr, pna)
-    zc, Gc, F, dF = pl["zc"], pl["Gc"], pl["F"], pl["dF"]
+    _, planes = sk.gr.build_cells(sl, PNA_PLANES if pna else PLUS_PLANES)
+    pl = _plus_planes(planes, pna)
+    zc, Gc = pl["zc"], pl["Gc"]
     emb, enc = _rule_embeddings(model, sl, dev)
     wts = [t.detach() for t in _tail_weights(model)]
-    if pna:                                                              # statistics -> scalers + Linear(12H,H) -> F holds y
-        ck.pna_stats(sl, emb, pl["pna"])
-        ck.pna_front_forward(sl, pl["pna"], wts[0], wts[1], F, pl["FEAT"], pl["SC"])
-    else:
-        ck.plus_features(sl, emb, F)
-    ck.tail_forward(sl, F, wts, zc, pl["bits"], front_done=pna)
+    _plus_scores(model, ck, sl, pl, emb, wts)
     ef = model.entity_feature
     ng = len(sl.group_sizes)
     extra = None
@@ -267,7 +293,7 @@ def plus_step(model, sk, sl, smoothing, grad_scale, gbuf: GradBuffer, expanded=F
             extra = model.RotatE.slot_scores(sk, sl)                               # dense by nature: [S][N][32]
         Z = extra.detach()
         ck.add_to_dense(sl, zc, Z)
-        loss, tsum, G = sk.softmax_ce(sl, Z, sl_dummy_mask(sl, sk), smoothing, False, sl.group_ptr_dev, ng, want_grad=want_grad)
+        loss, tsum, G = sk.softmax_ce(sl, Z, sl.nzmask, smoothing, False, sl.group_ptr_dev, ng, want_grad=want_grad)
         if want_grad:
             if grad_scale != 1.0:
                 G.mul_(grad_scale)
@@ -281,24 +307,15 @@ def plus_step(model, sk, sl, smoothing, grad_scale, gbuf: GradBuffer, expanded=F
     if not want_grad:
         return loss, tsum
     grads = [gbuf.view(p) for p in _tail_weights(model)]
-    ck.tail_backward(sl, model.num_relations, F, wts, Gc, pl["bits"], dF, pl["dY"], grads, model._d1sum_scratch(dev),
-                     front_done=pna)
-
-    def emb_backward(grad_emb):
-        if pna:
-            ck.pna_front_backward(sl, pl["pna"], wts[0], pl["dY"], pl["FEAT"], pl["SC"], pl["dstat"], grads[0])
-            ck.pna_backward(sl, emb, pl["pna"], pl["dstat"], grad_emb)
-        else:
-            ck.plus_backward(sl, dF, grad_emb)
-
     if model.type == "emb":
-        emb_backward(gbuf.view(model.rule_emb))
-    elif enc is not None:
+        gemb = gbuf.view(model.rule_emb)
+    else:
+        gemb = model._emb_scratch(dev, grad=True).zero_() if enc is not None else None
+    _plus_backward(model, ck, sl, pl, emb, wts, grads, gemb)
+    if enc is not None:
         ids, sub = enc
-        gfull = model._emb_scratch(dev, grad=True).zero_()
-        emb_backward(gfull)
         enc_params = [model.vocab_emb.weight] + [p for p in model.rnn.parameters()]
-        gs = torch.autograd.grad(sub, enc_params, gfull[ids].to(sub.dtype), allow_unused=True)
+        gs = torch.autograd.grad(sub, enc_params, gemb[ids].to(sub.dtype), allow_unused=True)
         for p, g_ in zip(enc_params, gs):
             if g_ is not None:
                 gbuf.view(p).add_(g_)
@@ -311,46 +328,128 @@ def plus_step(model, sk, sl, smoothing, grad_scale, gbuf: GradBuffer, expanded=F
     return loss, tsum
 
 
-def sl_dummy_mask(sl, sk):
-    """The dense CE kernels take a candidate-word table; with a dense entity feature the mask is all-true and
-    the table is never read (use_mask = 0) -- hand them the cells' own table."""
-    return _NzView(sl)
-
-
-class _NzView:
-    def __init__(self, sl):
-        self._p = sl.cells_tables["nzmask"]
-
-    def data_ptr(self):
-        return self._p
-
-
 @torch.no_grad()
 def plus_rank(model, sk, sl, split):
     ck = cell_kernels(sk)
     dev = sk.device
     sk.gr.ground(sl)
     pna = model.aggregator == "pna"
-    sk.gr.build_cells(sl, PNA_PLANES if pna else PLUS_PLANES)
-    pl = _plus_planes(sk.gr, pna)
-    zc, F = pl["zc"], pl["F"]
+    _, planes = sk.gr.build_cells(sl, PNA_PLANES if pna else PLUS_PLANES)
+    pl = _plus_planes(planes, pna)
+    zc = pl["zc"]
     emb, _ = _rule_embeddings(model, sl, dev)
-    wts = [t.detach() for t in _tail_weights(model)]
-    if pna:
-        ck.pna_stats(sl, emb, pl["pna"])
-        ck.pna_front_forward(sl, pl["pna"], wts[0], wts[1], F, pl["FEAT"], pl["SC"])
-    else:
-        ck.plus_features(sl, emb, F)
-    ck.tail_forward(sl, F, wts, zc, pl["bits"], front_done=pna)
+    _plus_scores(model, ck, sl, pl, emb, [t.detach() for t in _tail_weights(model)])
     which = "hr2oo" if split == "valid" else "hr2ooo"
     ef = model.entity_feature
     if ef == "RotatE":
         Z = model.RotatE.slot_scores(sk, sl).detach()
         ck.add_to_dense(sl, zc, Z)
-        return sk.filtered_rank(sl, Z, _NzView(sl), which, False)
+        return sk.filtered_rank(sl, Z, sl.nzmask, which, False)
     bias = model.bias.detach() if ef == "bias" else None
     sorted_bias = torch.sort(bias)[0] if bias is not None else None
     return ck.rank(sl, bias, sorted_bias, zc, which)
+
+
+# ================================================================================================
+# The reference's forward(all_h, all_r, edges_to_remove) -> (score [B,N], mask [B,N]) on the cells.  Two calls may be
+# alive before one backward(), so nothing here lives in the workspaces the fused steps reuse: the slots, the cell
+# arrays, the rule-embedding table and the gradients all belong to the call.
+# ================================================================================================
+def call_cells(sk, sl, floats_per_cell):
+    """rl_cells_build for a grounded API call into arrays of its own -> (planes, number of cells).  When the cells do
+    not fit, the frontier is expanded again and the cells built with exactly the count k_cell_scan reported."""
+    _, planes = sk.gr.build_cells(sl, floats_per_cell, cap=sk.gr.cell_capacity(sl))
+    n, over = sl.cell_counters[:2].tolist()
+    if over:
+        sk.gr._run(sl, sl.count_bits)
+        _, planes = sk.gr.build_cells(sl, floats_per_cell, cap=n)
+    return planes, n
+
+
+class _CellScoresFn(torch.autograd.Function):
+    """Cell scores of a Predictor (params: rule_weights) or a PredictorPlus (params: rule_emb or the encoder output of
+    the rules ``ids``, then the _tail_weights; none when the call has no cell) -> the reference's score [B,N]:
+    bias[e] (or the RotatE logits, or 0) + the cell's score, -inf outside the cells without an entity feature."""
+
+    @staticmethod
+    def forward(ctx, model, sk, sl, planes, ids, bias, extra, *params):
+        ck = cell_kernels(sk)
+        S, N = sl.S, sk.N
+        if extra is not None:
+            Z = extra.detach().clone()
+        elif bias is not None:
+            Z = bias.detach().view(1, N, 1).expand(S, N, LANES).contiguous()
+        else:
+            Z = torch.zeros(S, N, LANES, dtype=torch.float32, device=sk.device)
+        plus = hasattr(model, "score_model")
+        emb = wts = pl = None
+        if not plus:
+            ck.predictor_scores(sl, params[0].detach(), planes[0])
+            zc = planes[0]
+        elif params:
+            pl = _plus_planes(planes, model.aggregator == "pna")
+            emb = params[0].detach()
+            if ids is not None:                                          # encoder output -> table indexed by global rule id
+                emb = torch.zeros(model.num_rules, model.hidden_dim, dtype=torch.float32, device=sk.device).index_copy_(
+                    0, ids, emb.float())
+            wts = [t.detach() for t in params[1:]]
+            _plus_scores(model, ck, sl, pl, emb, wts)
+            zc = pl["zc"]
+        if not plus or params:
+            ck.add_to_dense(sl, zc, Z)
+        score, nz = sk.to_dense(sl, Z, sl.nzmask)
+        if bias is None and extra is None:
+            score.masked_fill_(~nz, float("-inf"))
+        ctx.model, ctx.sk, ctx.sl, ctx.planes, ctx.ids, ctx.pl, ctx.emb, ctx.wts = model, sk, sl, planes, ids, pl, emb, wts
+        ctx.has_bias, ctx.has_extra, ctx.params = bias is not None, extra is not None, [p.detach() for p in params]
+        ctx.mark_non_differentiable(nz)
+        return score, nz
+
+    @staticmethod
+    def backward(ctx, gscore, _gnz):
+        model, sk, sl, params = ctx.model, ctx.sk, ctx.sl, ctx.params
+        ck = cell_kernels(sk)
+        G = sk.from_dense(sl, gscore.contiguous())
+        grads = ()
+        if ctx.pl is None and params:                                    # Predictor
+            ck.gather_dense(sl, G, ctx.planes[1])
+            gw = torch.zeros_like(params[0])
+            ck.predictor_backward(sl, ctx.planes[1], gw)
+            grads = (gw,)
+        elif params:
+            ck.gather_dense(sl, G, ctx.pl["Gc"])
+            gt = [torch.zeros_like(p) for p in params[1:]]
+            gemb = torch.zeros_like(ctx.emb)
+            _plus_backward(model, ck, sl, ctx.pl, ctx.emb, ctx.wts, gt, gemb)
+            grads = (gemb if ctx.ids is None else gemb[ctx.ids].to(params[0].dtype),) + tuple(gt)
+        gb = G.sum(dim=(0, 2)) if ctx.has_bias else None
+        return (None, None, None, None, None, gb, G if ctx.has_extra else None) + grads
+
+
+def predictor_api_scores(model, sk, sl):
+    """Predictor.forward on a grounded call -> (score [B,N], nonzero mask [B,N], number of cells)."""
+    planes, n = call_cells(sk, sl, 2)                                    # zc, Gc
+    bias = model.bias if model.entity_feature == "bias" else None
+    score, nz = _CellScoresFn.apply(model, sk, sl, planes, None, bias, None, model.rule_weights)
+    return score, nz, n
+
+
+def plus_api_scores(model, sk, sl):
+    """PredictorPlus.forward on a grounded call (plus_cells_supported(model)) -> (score, nonzero mask, number of
+    cells).  Without a cell only the entity feature takes part (predictors.py:230-237)."""
+    planes, n = call_cells(sk, sl, PNA_PLANES if model.aggregator == "pna" else PLUS_PLANES)
+    ef = model.entity_feature
+    bias = model.bias if ef == "bias" else None
+    extra = model.RotatE.slot_scores(sk, sl) if ef == "RotatE" else None
+    ids, params = None, ()
+    if n > 0:
+        if model.type == "emb":
+            params = (model.rule_emb,) + tuple(_tail_weights(model))
+        else:
+            ids = _step_rule_ids(model, sl, sk.device)
+            params = (_encode_rules(model, ids),) + tuple(_tail_weights(model))
+    score, nz = _CellScoresFn.apply(model, sk, sl, planes, ids, bias, extra, *params)
+    return score, nz, n
 
 
 # ================================================================================================

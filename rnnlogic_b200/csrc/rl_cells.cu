@@ -27,15 +27,6 @@
 #include "rl_device.cuh"
 
 #define ITEM_GRID 8            // blocks per slot of the thread-per-item kernels
-#define PC_WARPS 4             // k_pred_cells / k_pred_cells_bwd (entity-grouped items, no coordinate list)
-#define PC_ROWS 4
-
-__device__ __forceinline__ uint32_t lanemask_lt()
-{
-    uint32_t m;
-    asm("mov.u32 %0, %%lanemask_lt;" : "=r"(m));
-    return m;
-}
 
 // order-preserving float <-> unsigned key (atomicMax on floats of either sign)
 __device__ __forceinline__ unsigned fkey(float v)
@@ -259,137 +250,6 @@ k_pred_zr_bwd(rl_graph g, rl_rules r, rl_slots s, rl_cells c, const float *__res
     v = warp_sum(v);
     if (lane == 0 && v != 0.0)
         for (int t = z0; t < z1; ++t) atomicAdd(grad_w + r.zr_rule[t], (float)v);
-}
-
-// ------------------------------------------------------------------------------------------
-// The same on the entity-grouped items (frontier with sort buffers; deterministic sums): one warp per 32 entities streams
-// the word's entity-grouped items, PC_ROWS count rows in flight; only the lanes of an item's mask touch its row.
-// ------------------------------------------------------------------------------------------
-template <typename CT>
-__global__ void __launch_bounds__(PC_WARPS * 32)
-k_pred_cells(rl_graph g, rl_rules r, rl_slots s, rl_frontier fr, rl_cells c, const float *__restrict__ w,
-             float *__restrict__ zc)
-{
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int slot = blockIdx.y;
-    const int ew = blockIdx.x * PC_WARPS + warp;
-    const int N = g.num_entities, W = g.rank_words;
-    if (ew >= W) return;
-    const int e_lane = ew * 32 + lane;
-    const uint32_t my_bits = e_lane < N ? c.nzmask[(size_t)slot * N + e_lane] : 0u;
-    if (__ballot_sync(FULL, my_bits != 0u) == 0u) return;
-    const int my_off = e_lane < N ? c.cand_off[(size_t)slot * N + e_lane] : 0;
-    const int q = s.slot_head[slot];
-    const CT *arena = reinterpret_cast<const CT *>(fr.arena) + (size_t)s.arena_off[slot] * RL_LANES;
-    const int h = s.lane_h[slot * RL_LANES + lane];
-    const int z0 = r.zr_ptr[q], z1 = r.zr_ptr[q + 1];
-    double zsum = 0.0;
-    for (int t = z0; t < z1; ++t) zsum += (double)__ldg(w + r.zr_rule[t]);
-    const uint32_t lt = lanemask_lt();
-    auto finish = [&](int i, double acc) {
-        if (z1 > z0 && h == ew * 32 + i) acc += zsum;         // empty-body rules: count = one_hot(h)
-        const uint32_t bits = __shfl_sync(FULL, my_bits, i);
-        const int off = __shfl_sync(FULL, my_off, i);
-        if ((bits >> lane) & 1u) {
-            const int idx = off + __popc(bits & lt);
-            if (idx < c.cap) zc[idx] = (float)acc;
-        }
-    };
-    WordItems wi = load_word_items(fr, s, W, slot, ew);
-    int cur = -1;
-    double acc = 0.0;
-    const int B0 = __shfl_sync(FULL, wi.b0, 0), B1 = wi.wend;
-    for (int c0 = B0; c0 < B1; c0 += 32) {
-        if (c0 != wi.wbase) word_items_window(wi, c0);
-        const int cnt = min(32, B1 - c0);
-        for (int j0 = 0; j0 < cnt; j0 += PC_ROWS) {
-            CT cv[PC_ROWS];
-            float wv[PC_ROWS];
-#pragma unroll
-            for (int u = 0; u < PC_ROWS; ++u) {
-                const int src = (j0 + u) & 31;
-                const int a = __shfl_sync(FULL, wi.win.x, src);
-                const int t0 = __shfl_sync(FULL, wi.win.y, src);
-                const uint32_t m = __shfl_sync(FULL, wi.wmask, src);
-                const bool ok = j0 + u < cnt;
-                cv[u] = (ok && ((m >> lane) & 1u)) ? arena[(size_t)a * RL_LANES + lane] : (CT)0;
-                wv[u] = ok ? __ldg(w + __ldg(r.node_term_rule + t0)) : 0.f;
-            }
-#pragma unroll
-            for (int u = 0; u < PC_ROWS; ++u) {
-                if (j0 + u >= cnt) break;
-                const int src = (j0 + u) & 31;
-                const int i = __shfl_sync(FULL, wi.win.z, src) & 31;
-                const int nt = __shfl_sync(FULL, wi.win.w, src);
-                if (i != cur) {
-                    if (cur >= 0) finish(cur, acc);
-                    cur = i;
-                    acc = 0.0;
-                }
-                const double cf = (double)(float)cv[u];                                // x.float() * w (predictors.py:64)
-                acc += cf * (double)wv[u];
-                if (nt > 1) {                                                          // duplicate rules ending at the same node
-                    const int t0 = __shfl_sync(FULL, wi.win.y, src);
-                    for (int t = t0 + 1; t < t0 + nt; ++t) acc += cf * (double)__ldg(w + r.node_term_rule[t]);
-                }
-            }
-        }
-    }
-    if (cur >= 0) finish(cur, acc);
-    const uint32_t present = __ballot_sync(FULL, my_bits != 0u);
-    for (uint32_t todo = present & ~wi.present; todo; todo &= todo - 1) finish(__ffs(todo) - 1, 0.0);   // cells of empty-body rules only
-}
-
-template <typename CT>
-__global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, 4)
-k_pred_cells_bwd(rl_graph g, rl_rules r, rl_slots s, rl_frontier fr, rl_cells c, const float *__restrict__ Gc,
-                 float *__restrict__ grad_w)
-{
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int slot = blockIdx.y;
-    const int ew = blockIdx.x * WARPS_PER_BLOCK + warp;
-    const int N = g.num_entities, W = g.rank_words;
-    const size_t srow = (size_t)slot * N;
-    if (ew >= W) return;
-    const int e_lane = ew * 32 + lane;
-    const uint32_t my_bits = e_lane < N ? c.nzmask[srow + e_lane] : 0u;
-    if (__ballot_sync(FULL, my_bits != 0u) == 0u) return;
-    const int my_off = e_lane < N ? c.cand_off[srow + e_lane] : 0;
-    const CT *arena = reinterpret_cast<const CT *>(fr.arena) + (size_t)s.arena_off[slot] * RL_LANES;
-    const uint32_t lt = lanemask_lt();
-    WordItems wi = load_word_items(fr, s, W, slot, ew);
-    const int B0 = __shfl_sync(FULL, wi.b0, 0), B1 = wi.wend;
-    for (int c0 = B0; c0 < B1; c0 += 32) {
-        if (c0 != wi.wbase) word_items_window(wi, c0);
-        const int cnt = min(32, B1 - c0);
-        for (int j0 = 0; j0 < cnt; j0 += BWD_ROWS) {
-            float pv[BWD_ROWS];
-#pragma unroll
-            for (int u = 0; u < BWD_ROWS; ++u) {
-                const int src = (j0 + u) & 31;
-                const int a = __shfl_sync(FULL, wi.win.x, src);
-                const int i = __shfl_sync(FULL, wi.win.z, src) & 31;
-                const uint32_t m = __shfl_sync(FULL, wi.wmask, src);
-                const uint32_t bits = __shfl_sync(FULL, my_bits, i);
-                const int off = __shfl_sync(FULL, my_off, i);
-                pv[u] = 0.f;
-                if (j0 + u < cnt && ((m >> lane) & 1u)) {          // a non-zero count => the cell exists
-                    const int idx = off + __popc(bits & lt);
-                    const CT cv = arena[(size_t)a * RL_LANES + lane];
-                    if (idx < c.cap) pv[u] = (float)cv * Gc[idx];
-                }
-            }
-#pragma unroll
-            for (int u = 0; u < BWD_ROWS; ++u) {
-                if (j0 + u >= cnt) break;
-                const float v = warp_sumf(pv[u]);
-                const int src = (j0 + u) & 31;
-                const int t0 = __shfl_sync(FULL, wi.win.y, src), nt = __shfl_sync(FULL, wi.win.w, src);
-                if (lane == 0 && v != 0.f)
-                    for (int t = t0; t < t0 + nt; ++t) atomicAdd(grad_w + r.node_term_rule[t], v);
-            }
-        }
-    }
 }
 
 // ------------------------------------------------------------------------------------------
@@ -694,7 +554,7 @@ k_rank_cells_finalize(rl_graph g, rl_slots s, rl_cells c, rl_answers known, cons
 }
 
 // ------------------------------------------------------------------------------------------
-// cells <-> dense entity-major matrices (the RotatE entity feature is dense by nature; API forward())
+// cells <-> dense entity-major matrices (the RotatE entity feature is dense by nature; the [B,N] scores of forward())
 // ------------------------------------------------------------------------------------------
 // mode 0: Z[cell position] += zc     mode 1: Gc = G[cell position]
 __global__ void __launch_bounds__(256)
@@ -720,11 +580,6 @@ static int bad_item_frontier(const rl_frontier *fr)
     return !fr || !fr->arena || !fr->items || !fr->item_cnt || !fr->item_off || !fr->nzmask ||
            (fr->count_bits != 32 && fr->count_bits != 64);
 }
-static int no_sorted(const rl_frontier *fr)
-{
-    return !fr->items_sorted || !fr->bucket_cnt || !fr->bucket_off || !fr->item_mask || !fr->item_mask_sorted;
-}
-
 extern "C" {
 
 int rl_cells_build(const rl_graph *g, const rl_rules *r, const rl_slots *s, const rl_frontier *fr,
@@ -735,11 +590,8 @@ int rl_cells_build(const rl_graph *g, const rl_rules *r, const rl_slots *s, cons
     if ((c->qmax == nullptr) != (c->qsum == nullptr)) return rl_fail(RL_ERR_ARG, "rl_cells_build: qmax and qsum go together");
     if (s->num_slots <= 0) return RL_OK;
     if (!fr->item_mask) return rl_fail(RL_ERR_ARG, "rl_cells_build: the frontier was expanded without lane masks");
-    if (fr->bucket_cnt) {                                         // sort buffers: the candidate words come from the sort
-        if (no_sorted(fr)) return rl_fail(RL_ERR_ARG, "rl_cells_build: incomplete sort buffers");
-        const int rc = rl_sort_items(g, s, fr, stream);           // groups items by entity, ORs their lane masks into nzmask
-        if (rc != RL_OK) return rc;
-    }
+    if (fr->bucket_cnt)                                           // the sort, not k_numeric, fills nzmask of such a frontier
+        return rl_fail(RL_ERR_ARG, "rl_cells_build: the frontier has sort buffers; expand it without bucket tables");
     k_cell_scan<<<s->num_slots, 512, 0, (cudaStream_t)stream>>>(*g, *r, *s, *c);
     CHECK_LAUNCH("k_cell_scan");
     return RL_OK;
@@ -784,38 +636,6 @@ int rl_predictor_item_backward(const rl_graph *g, const rl_rules *r, const rl_sl
     if (fr->count_bits == 32) k_pred_item_bwd<uint32_t><<<grid, 256, 0, st>>>(*g, *r, *s, *fr, *c, Gc, grad_w);
     else k_pred_item_bwd<unsigned long long><<<grid, 256, 0, st>>>(*g, *r, *s, *fr, *c, Gc, grad_w);
     CHECK_LAUNCH("k_pred_item_bwd");
-    if (r->num_zero_rules > 0) {
-        k_pred_zr_bwd<<<s->num_slots, 32, 0, st>>>(*g, *r, *s, *c, Gc, grad_w);
-        CHECK_LAUNCH("k_pred_zr_bwd");
-    }
-    return RL_OK;
-}
-
-int rl_predictor_cell_scores(const rl_graph *g, const rl_rules *r, const rl_slots *s, const rl_frontier *fr,
-                             const rl_cells *c, const float *w, float *zc, void *stream)
-{
-    if (!g || !r || !s || !w || !zc || bad_cells(c) || bad_item_frontier(fr) || no_sorted(fr))
-        return rl_fail(RL_ERR_ARG, "rl_predictor_cell_scores: bad argument");
-    if (s->num_slots <= 0) return RL_OK;
-    const dim3 grid((g->rank_words + PC_WARPS - 1) / PC_WARPS, s->num_slots);
-    cudaStream_t st = (cudaStream_t)stream;
-    if (fr->count_bits == 32) k_pred_cells<uint32_t><<<grid, PC_WARPS * 32, 0, st>>>(*g, *r, *s, *fr, *c, w, zc);
-    else k_pred_cells<unsigned long long><<<grid, PC_WARPS * 32, 0, st>>>(*g, *r, *s, *fr, *c, w, zc);
-    CHECK_LAUNCH("k_pred_cells");
-    return RL_OK;
-}
-
-int rl_predictor_cell_backward(const rl_graph *g, const rl_rules *r, const rl_slots *s, const rl_frontier *fr,
-                               const rl_cells *c, const float *Gc, float *grad_w, void *stream)
-{
-    if (!g || !r || !s || !Gc || !grad_w || bad_cells(c) || bad_item_frontier(fr) || no_sorted(fr))
-        return rl_fail(RL_ERR_ARG, "rl_predictor_cell_backward: bad argument");
-    if (s->num_slots <= 0) return RL_OK;
-    const dim3 grid((g->rank_words + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK, s->num_slots);
-    cudaStream_t st = (cudaStream_t)stream;
-    if (fr->count_bits == 32) k_pred_cells_bwd<uint32_t><<<grid, WARPS_PER_BLOCK * 32, 0, st>>>(*g, *r, *s, *fr, *c, Gc, grad_w);
-    else k_pred_cells_bwd<unsigned long long><<<grid, WARPS_PER_BLOCK * 32, 0, st>>>(*g, *r, *s, *fr, *c, Gc, grad_w);
-    CHECK_LAUNCH("k_pred_cells_bwd");
     if (r->num_zero_rules > 0) {
         k_pred_zr_bwd<<<s->num_slots, 32, 0, st>>>(*g, *r, *s, *c, Gc, grad_w);
         CHECK_LAUNCH("k_pred_zr_bwd");

@@ -879,54 +879,7 @@ k_grad_sparse(rl_graph g, rl_slots s, rl_answers ans, float smoothing, int use_m
 // ------------------------------------------------------------------------------------------
 // kernel (2c): backward into rule weights / bias
 // ------------------------------------------------------------------------------------------
-// Backward over the item list: one warp per non-zero terminal row: <G[e], fp32(count row)> goes to
-// every rule ending at the row's node (one atomic each).
-#define ITEM_BLOCKS 96
-// sorted != 0: walk the entity-grouped list (after rl_sort_items) -- neighbouring warps then share rows of G.
-template <typename CT>
-__global__ void __launch_bounds__(WARPS_PER_BLOCK * 32)
-k_predictor_bwd_items(rl_graph g, rl_rules r, rl_slots s, rl_frontier fr, const float *__restrict__ G,
-                      const float *__restrict__ slot_scale, float *__restrict__ grad_w, int sorted)
-{
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int slot = blockIdx.y;
-    const int n = fr.item_cnt[slot];
-    const int N = g.num_entities;
-    const int q = s.slot_head[slot];
-    const float scale = slot_scale ? slot_scale[slot] : 1.f;
-    const float *Gs = G + (size_t)slot * N * RL_LANES;
-    auto grad_at = [&](int e) -> float { return Gs[(size_t)e * RL_LANES + lane]; };
-    const int z0 = r.zr_ptr[q], z1 = r.zr_ptr[q + 1];
-    if (blockIdx.x == 0 && warp == 0 && z1 > z0) {                 // empty-body rules: count = one_hot(h)
-        const int h = s.lane_h[slot * RL_LANES + lane];
-        double v = h >= 0 ? (double)grad_at(h) : 0.0;
-        v = warp_sum(v);
-        if (lane == 0)
-            for (int t = z0; t < z1; ++t) atomicAdd(grad_w + r.zr_rule[t], (float)v * scale);
-    }
-    const CT *arena = reinterpret_cast<const CT *>(fr.arena) + (size_t)s.arena_off[slot] * RL_LANES;
-    const int4 *it = reinterpret_cast<const int4 *>(sorted ? fr.items_sorted : fr.items) + fr.item_off[slot];
-    const int stride = ITEM_BLOCKS * WARPS_PER_BLOCK;
-    for (int i = blockIdx.x * WARPS_PER_BLOCK + warp; i < n; i += 2 * stride) {     // two items in flight
-        const int i2 = i + stride;
-        const int4 ra = __ldg(it + i);                             // {row, first rule end, entity, rule ends}
-        const int4 rb = i2 < n ? __ldg(it + i2) : ra;
-        const CT ca = arena[(size_t)ra.x * RL_LANES + lane];
-        const CT cb = arena[(size_t)rb.x * RL_LANES + lane];
-        const float ga = grad_at(ra.z);
-        const float gb = grad_at(rb.z);
-        double va = ca != 0 ? (double)(float)ca * (double)ga : 0.0;     // skips NaN*0 of masked cells
-        double vb = (i2 < n && cb != 0) ? (double)(float)cb * (double)gb : 0.0;
-        va = warp_sum(va);
-        vb = warp_sum(vb);
-        if (lane == 0 && va != 0.0)
-            for (int t = ra.y; t < ra.y + ra.w; ++t) atomicAdd(grad_w + r.node_term_rule[t], (float)va * scale);
-        if (lane == 0 && vb != 0.0)
-            for (int t = rb.y; t < rb.y + rb.w; ++t) atomicAdd(grad_w + r.node_term_rule[t], (float)vb * scale);
-    }
-}
-
-// The same backward over the entity-grouped list (after rl_sort_items): one warp per 32 entities streams
+// Backward over the entity-grouped item list (after rl_sort_items): one warp per 32 entities streams
 // the word's items four at a time (count row + G row of each in flight together; items of one entity hit
 // the same G row), fp32 products as the reference's x.float() * grad, one warp reduction per item.
 template <typename CT>
@@ -981,21 +934,7 @@ k_predictor_bwd_stream(rl_graph g, rl_rules r, rl_slots s, rl_frontier fr, const
     }
 }
 
-__global__ void __launch_bounds__(WARPS_PER_BLOCK * 32)
-k_bias_grad(int N, int S, const float *__restrict__ G, const float *__restrict__ slot_scale,
-            float *__restrict__ grad_bias)
-{
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int e = blockIdx.x * WARPS_PER_BLOCK + warp;
-    if (e >= N) return;
-    double acc = 0.0;
-    for (int sl = 0; sl < S; ++sl)
-        acc += (double)G[((size_t)sl * N + e) * RL_LANES + lane] * (double)(slot_scale ? slot_scale[sl] : 1.f);
-    acc = warp_sum(acc);
-    if (lane == 0) grad_bias[e] += (float)acc;
-}
-
-// k_grad_dense and the dense part of k_bias_grad in one sweep over Z: a warp owns BIAS_ROWS consecutive
+// k_grad_dense and the dense part of the bias gradient in one sweep over Z: a warp owns BIAS_ROWS consecutive
 // entities (1 KB of contiguous logits per slot) and loops over slots, so the per-query (max, coefficient)
 // pair is loaded once per slot and warp instead of once per row; G[sl][e][b] = coef_b * exp(z - max_b) is
 // written and summed into grad_bias[e] on the way.
@@ -1415,23 +1354,6 @@ int rl_softmax_ce(const rl_graph *g, const rl_slots *s, const rl_answers *ans, f
     return RL_OK;
 }
 
-static int launch_bwd_items(const rl_graph *g, const rl_rules *r, const rl_slots *s, const rl_frontier *fr, const float *G,
-                            const float *slot_scale, float *grad_w, int sorted, cudaStream_t st)
-{
-    if (sorted) {
-        const dim3 grid((g->rank_words + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK, s->num_slots);
-        if (fr->count_bits == 32) k_predictor_bwd_stream<uint32_t><<<grid, WARPS_PER_BLOCK * 32, 0, st>>>(*g, *r, *s, *fr, G, slot_scale, grad_w);
-        else k_predictor_bwd_stream<unsigned long long><<<grid, WARPS_PER_BLOCK * 32, 0, st>>>(*g, *r, *s, *fr, G, slot_scale, grad_w);
-        CHECK_LAUNCH("k_predictor_bwd_stream");
-        return RL_OK;
-    }
-    const dim3 grid(ITEM_BLOCKS, s->num_slots);
-    if (fr->count_bits == 32) k_predictor_bwd_items<uint32_t><<<grid, WARPS_PER_BLOCK * 32, 0, st>>>(*g, *r, *s, *fr, G, slot_scale, grad_w, 0);
-    else k_predictor_bwd_items<unsigned long long><<<grid, WARPS_PER_BLOCK * 32, 0, st>>>(*g, *r, *s, *fr, G, slot_scale, grad_w, 0);
-    CHECK_LAUNCH("k_predictor_bwd_items");
-    return RL_OK;
-}
-
 int rl_predictor_ce_backward(const rl_graph *g, const rl_rules *r, const rl_slots *s, const rl_frontier *fr,
                              const rl_answers *ans, float smoothing, int32_t use_mask, const float *Z,
                              const uint32_t *nzmask, int32_t n_groups, const int32_t *group_ptr, float *partial,
@@ -1462,24 +1384,10 @@ int rl_predictor_ce_backward(const rl_graph *g, const rl_rules *r, const rl_slot
     }
     k_grad_sparse<<<S, CE_WARPS * 32, 0, st>>>(*g, *s, *ans, smoothing, use_mask, Z, nzmask, stats, slot_invT, G, slot_scale, grad_bias);
     CHECK_LAUNCH("k_grad_sparse");
-    return launch_bwd_items(g, r, s, fr, G, slot_scale, grad_w, 1, st);
-}
-
-int rl_predictor_backward(const rl_graph *g, const rl_rules *r, const rl_slots *s, const rl_frontier *fr,
-                          const float *G, const float *slot_scale, float *grad_w, float *grad_bias, void *stream)
-{
-    if (!g || !r || !s || !G || !grad_w) return fail(RL_ERR_ARG, "rl_predictor_backward: null argument");
-    if (check_frontier(fr, "rl_predictor_backward: incomplete rl_frontier") != RL_OK) return RL_ERR_ARG;
-    if (check_items(fr, "rl_predictor_backward: the frontier was expanded without an item list") != RL_OK) return RL_ERR_ARG;
-    const int S = s->num_slots, N = g->num_entities;
-    if (S <= 0) return RL_OK;
-    cudaStream_t st = (cudaStream_t)stream;
-    const int rc = launch_bwd_items(g, r, s, fr, G, slot_scale, grad_w, 0, st);
-    if (rc != RL_OK) return rc;
-    if (grad_bias) {
-        k_bias_grad<<<(N + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK, WARPS_PER_BLOCK * 32, 0, st>>>(N, S, G, slot_scale, grad_bias);
-        CHECK_LAUNCH("k_bias_grad");
-    }
+    const dim3 grid((g->rank_words + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK, S);
+    if (fr->count_bits == 32) k_predictor_bwd_stream<uint32_t><<<grid, WARPS_PER_BLOCK * 32, 0, st>>>(*g, *r, *s, *fr, G, slot_scale, grad_w);
+    else k_predictor_bwd_stream<unsigned long long><<<grid, WARPS_PER_BLOCK * 32, 0, st>>>(*g, *r, *s, *fr, G, slot_scale, grad_w);
+    CHECK_LAUNCH("k_predictor_bwd_stream");
     return RL_OK;
 }
 

@@ -271,222 +271,7 @@ k_rule_stats(rl_graph g, rl_rules r, rl_slots s, rl_frontier fr, int max_terms, 
 // Cells are numbered by rl_cells_build before any count row is read again (the candidate words come from the
 // items' lane masks), so one pass over the count rows produces the aggregates at their final place.
 // ==========================================================================================
-#define PCELL_WARPS 4
-#define PCELL_ROWS 4
 #define CH 16                                                     // hidden_dim of the cell kernels
-
-__device__ __forceinline__ uint32_t plus_lanemask_lt()
-{
-    uint32_t m;
-    asm("mov.u32 %0, %%lanemask_lt;" : "=r"(m));
-    return m;
-}
-
-// F[cell][16] = sum_rule fp32(count) * emb[rule]  (layers.py:68-72); emb is indexed by the GLOBAL rule id.
-// PNA adds sum count*emb^2, min / max over rules with a non-zero count + their arg rules, degree (layers.py:92-99).
-template <typename CT, bool PNA>
-__global__ void __launch_bounds__(PCELL_WARPS * 32)
-k_plus_cells(rl_graph g, rl_rules r, rl_slots s, rl_frontier fr, rl_cells c, const float *__restrict__ emb,
-             float *__restrict__ out_sum, float *__restrict__ out_sq, float *__restrict__ out_min,
-             float *__restrict__ out_max, int32_t *__restrict__ arg_min, int32_t *__restrict__ arg_max,
-             float *__restrict__ degree)
-{
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int slot = blockIdx.y;
-    const int ew = blockIdx.x * PCELL_WARPS + warp;
-    const int N = g.num_entities, W = g.rank_words;
-    if (ew >= W) return;
-    const int e_lane = ew * 32 + lane;
-    const uint32_t my_bits = e_lane < N ? c.nzmask[(size_t)slot * N + e_lane] : 0u;
-    const uint32_t present = __ballot_sync(FULL, my_bits != 0u);
-    if (present == 0u) return;
-    const int my_off = e_lane < N ? c.cand_off[(size_t)slot * N + e_lane] : 0;
-    const int q = s.slot_head[slot];
-    const CT *arena = reinterpret_cast<const CT *>(fr.arena) + (size_t)s.arena_off[slot] * RL_LANES;
-    const int h = s.lane_h[slot * RL_LANES + lane];
-    const int z0 = r.zr_ptr[q], z1 = r.zr_ptr[q + 1];
-    const uint32_t lt = plus_lanemask_lt();
-    double a1[CH], a2[PNA ? CH : 1];
-    float mn[PNA ? CH : 1], mx[PNA ? CH : 1];
-    int amn[PNA ? CH : 1], amx[PNA ? CH : 1];
-    double deg = 1.0;
-    auto reset = [&]() {
-        deg = 1.0;
-#pragma unroll
-        for (int k = 0; k < CH; ++k) {
-            a1[k] = 0.0;
-            if (PNA) { a2[k] = 0.0; mn[k] = INFINITY; mx[k] = -INFINITY; amn[k] = -1; amx[k] = -1; }
-        }
-    };
-    auto add = [&](float cf, int rule) {                          // called by the lanes with a non-zero count only
-        const float4 *er = reinterpret_cast<const float4 *>(emb + (size_t)rule * CH);
-        deg += (double)cf;
-#pragma unroll
-        for (int k4 = 0; k4 < CH / 4; ++k4) {
-            const float4 v4 = __ldg(er + k4);
-            const float ev[4] = {v4.x, v4.y, v4.z, v4.w};
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                const int k = 4 * k4 + u;
-                a1[k] += (double)cf * (double)ev[u];
-                if (PNA) {
-                    a2[k] += (double)cf * (double)(ev[u] * ev[u]);
-                    if (ev[u] < mn[k]) { mn[k] = ev[u]; amn[k] = rule; }
-                    if (ev[u] > mx[k]) { mx[k] = ev[u]; amx[k] = rule; }
-                }
-            }
-        }
-    };
-    auto finish = [&](int i) {
-        const int e = ew * 32 + i;
-        if (z1 > z0 && h == e)                                    // empty-body rules: count = one_hot(h)
-            for (int t = z0; t < z1; ++t) add(1.f, r.zr_rule[t]);
-        const uint32_t bits = __shfl_sync(FULL, my_bits, i);
-        const int off = __shfl_sync(FULL, my_off, i);
-        if ((bits >> lane) & 1u) {
-            const long long idx = off + __popc(bits & lt);
-            if (idx < c.cap) {
-                float4 *o = reinterpret_cast<float4 *>(out_sum + idx * CH);
-#pragma unroll
-                for (int k4 = 0; k4 < CH / 4; ++k4)
-                    o[k4] = make_float4((float)a1[4 * k4], (float)a1[4 * k4 + 1], (float)a1[4 * k4 + 2], (float)a1[4 * k4 + 3]);
-                if (PNA) {
-#pragma unroll
-                    for (int k = 0; k < CH; ++k) {
-                        out_sq[idx * CH + k] = (float)a2[k];
-                        out_min[idx * CH + k] = mn[k];
-                        out_max[idx * CH + k] = mx[k];
-                        arg_min[idx * CH + k] = amn[k];
-                        arg_max[idx * CH + k] = amx[k];
-                    }
-                    degree[idx] = (float)deg;
-                }
-            }
-        }
-        reset();
-    };
-    reset();
-    WordItems wi = load_word_items(fr, s, W, slot, ew);
-    int cur = -1;
-    const int B0 = __shfl_sync(FULL, wi.b0, 0), B1 = wi.wend;
-    for (int c0 = B0; c0 < B1; c0 += 32) {
-        if (c0 != wi.wbase) word_items_window(wi, c0);
-        const int cnt = min(32, B1 - c0);
-        for (int j0 = 0; j0 < cnt; j0 += PCELL_ROWS) {
-            CT cv[PCELL_ROWS];
-#pragma unroll
-            for (int u = 0; u < PCELL_ROWS; ++u) {
-                const int src = (j0 + u) & 31;
-                const int a = __shfl_sync(FULL, wi.win.x, src);
-                const uint32_t m = __shfl_sync(FULL, wi.wmask, src);
-                cv[u] = (j0 + u < cnt && ((m >> lane) & 1u)) ? arena[(size_t)a * RL_LANES + lane] : (CT)0;
-            }
-#pragma unroll
-            for (int u = 0; u < PCELL_ROWS; ++u) {
-                if (j0 + u >= cnt) break;
-                const int src = (j0 + u) & 31;
-                const int i = __shfl_sync(FULL, wi.win.z, src) & 31;
-                const int t0 = __shfl_sync(FULL, wi.win.y, src);
-                const int nt = __shfl_sync(FULL, wi.win.w, src);
-                if (i != cur) {
-                    if (cur >= 0) finish(cur);
-                    cur = i;
-                }
-                if (cv[u] != 0) {
-                    const float cf = (float)cv[u];
-                    for (int t = t0; t < t0 + nt; ++t) add(cf, __ldg(r.node_term_rule + t));
-                }
-            }
-        }
-    }
-    if (cur >= 0) finish(cur);
-    for (uint32_t todo = present & ~wi.present; todo; todo &= todo - 1) finish(__ffs(todo) - 1);   // cells of empty-body rules only
-}
-
-// Backward into the rule embeddings: gEmb[rule][:] += sum over (row, query) of fp32(count) * dF[cell][:].
-// Walks the UNSORTED item list, where the <= 32 rows one k_numeric tile appended are consecutive and belong to
-// one trie node: a warp takes 32 consecutive items, accumulates while the node stays the same (lanes = 2 cells x
-// 16 hidden units) and issues one atomic per hidden unit and rule ending at the node per run.
-#define PCB_BLOCKS 64
-template <typename CT>
-__global__ void __launch_bounds__(WARPS_PER_BLOCK * 32)
-k_plus_cells_bwd(rl_graph g, rl_rules r, rl_slots s, rl_frontier fr, rl_cells c, const float *__restrict__ dF,
-                 float *__restrict__ gEmb)
-{
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int slot = blockIdx.y;
-    const int N = g.num_entities;
-    const int q = s.slot_head[slot];
-    const size_t srow = (size_t)slot * N;
-    const int half = lane >> 4, hh = lane & 15;
-    if (blockIdx.x == 0 && warp == 0 && r.zr_ptr[q + 1] > r.zr_ptr[q]) {       // empty-body rules: count = one_hot(h)
-        const int hq = s.lane_h[slot * RL_LANES + lane];
-        long long my_idx = -1;
-        if (hq >= 0) {
-            const uint32_t bits = c.nzmask[srow + hq];
-            const long long idx = c.cand_off[srow + hq] + __popc(bits & ((1u << lane) - 1u));
-            if (((bits >> lane) & 1u) && idx < c.cap) my_idx = idx;
-        }
-        float acc = 0.f;
-        for (int b = half; b < 32; b += 2) {
-            const long long idx = __shfl_sync(FULL, my_idx, b);
-            if (idx >= 0) acc += dF[idx * CH + hh];
-        }
-        acc += __shfl_xor_sync(FULL, acc, 16);
-        if (half == 0 && acc != 0.f)
-            for (int t = r.zr_ptr[q]; t < r.zr_ptr[q + 1]; ++t) atomicAdd(gEmb + (size_t)r.zr_rule[t] * CH + hh, acc);
-    }
-    const int n = fr.item_cnt[slot];
-    const CT *arena = reinterpret_cast<const CT *>(fr.arena) + (size_t)s.arena_off[slot] * RL_LANES;
-    const int4 *items = reinterpret_cast<const int4 *>(fr.items) + fr.item_off[slot];
-    const uint32_t *masks = fr.item_mask + fr.item_off[slot];
-    for (int base = (blockIdx.x * WARPS_PER_BLOCK + warp) * 32; base < n; base += PCB_BLOCKS * WARPS_PER_BLOCK * 32) {
-        const int cnt = min(32, n - base);
-        int4 it = make_int4(0, -1, 0, 0);
-        uint32_t m = 0u, bits = 0u;
-        int off = 0;
-        if (lane < cnt) {
-            it = __ldg(items + base + lane);                      // {row, first rule end, entity, rule ends}
-            m = __ldg(masks + base + lane);
-            bits = c.nzmask[srow + it.z];
-            off = c.cand_off[srow + it.z];
-        }
-        int cur_t0 = -1, cur_nt = 0;
-        float acc = 0.f;
-        auto flush = [&]() {
-            acc += __shfl_xor_sync(FULL, acc, 16);
-            if (cur_t0 >= 0 && half == 0 && acc != 0.f)
-                for (int t = cur_t0; t < cur_t0 + cur_nt; ++t) atomicAdd(gEmb + (size_t)__ldg(r.node_term_rule + t) * CH + hh, acc);
-            acc = 0.f;
-        };
-        for (int j = 0; j < cnt; ++j) {
-            const int row = __shfl_sync(FULL, it.x, j), t0 = __shfl_sync(FULL, it.y, j), nt = __shfl_sync(FULL, it.w, j);
-            uint32_t mj = __shfl_sync(FULL, m, j);
-            const uint32_t bj = __shfl_sync(FULL, bits, j);
-            const int oj = __shfl_sync(FULL, off, j);
-            if (t0 != cur_t0) {
-                flush();
-                cur_t0 = t0;
-                cur_nt = nt;
-            }
-            const CT cv = ((mj >> lane) & 1u) ? arena[(size_t)row * RL_LANES + lane] : (CT)0;
-            while (mj) {                                          // two non-zero queries per pass, one per half warp
-                const int b0 = __ffs(mj) - 1;
-                mj &= mj - 1;
-                const int b1 = mj ? __ffs(mj) - 1 : -1;
-                mj &= mj - 1;
-                const float c0v = (float)__shfl_sync(FULL, cv, b0);
-                const float c1v = (float)__shfl_sync(FULL, cv, b1 & 31);
-                const int b = half ? b1 : b0;
-                if (b >= 0) {
-                    const long long idx = oj + __popc(bj & ((1u << b) - 1u));
-                    if (idx < c.cap) acc = fmaf(half ? c1v : c0v, dF[idx * CH + hh], acc);
-                }
-            }
-        }
-        flush();
-    }
-}
 
 // ---- PredictorPlus on the item list as k_numeric appended it: one thread per (item, quarter of the hidden vector) ----
 #define PN_BLOCKS 16
@@ -610,6 +395,12 @@ static int bad_frontier(const rl_frontier *fr)
            !fr->bucket_cnt || !fr->bucket_off || (fr->count_bits != 32 && fr->count_bits != 64);
 }
 
+static int no_item_arg(const rl_frontier *fr)
+{
+    return !fr || !fr->arena || !fr->items || !fr->item_off || !fr->item_cnt || !fr->item_mask ||
+           (fr->count_bits != 32 && fr->count_bits != 64);
+}
+
 extern "C" {
 
 int rl_plus_mask(const rl_graph *g, const rl_rules *r, const rl_slots *s, const rl_frontier *fr, uint32_t *nzmask,
@@ -651,7 +442,7 @@ int rl_plus_features(const rl_graph *g, const rl_rules *r, const rl_slots *s, co
 int rl_rule_stats(const rl_graph *g, const rl_rules *r, const rl_slots *s, const rl_frontier *fr, int32_t max_terms,
                   double *sum_cnt, double *pos_cnt, void *stream)
 {
-    if (!g || !r || !s || !sum_cnt || !pos_cnt || bad_frontier(fr) || max_terms <= 0) return rl_fail(RL_ERR_ARG, "rl_rule_stats: bad argument");
+    if (!g || !r || !s || !sum_cnt || !pos_cnt || no_item_arg(fr) || max_terms <= 0) return rl_fail(RL_ERR_ARG, "rl_rule_stats: bad argument");
     if (s->num_slots <= 0) return RL_OK;
     dim3 grid(PLUS_ITEM_BLOCKS, s->num_slots);
     cudaStream_t st = (cudaStream_t)stream;
@@ -688,47 +479,6 @@ int rl_plus_gather(const rl_graph *g, const rl_slots *s, const uint32_t *nzmask,
 static int bad_cells_arg(const rl_cells *c)
 {
     return !c || !c->counters || !c->nzmask || !c->cand_off || !c->cell_key || c->cap <= 0;
-}
-
-int rl_plus_cell_features(const rl_graph *g, const rl_rules *r, const rl_slots *s, const rl_frontier *fr,
-                          const rl_cells *c, const float *emb, int32_t H, int32_t pna, float *out_sum, float *out_sq,
-                          float *out_min, float *out_max, int32_t *arg_min, int32_t *arg_max, float *degree, void *stream)
-{
-    if (!g || !r || !s || !emb || !out_sum || bad_frontier(fr) || bad_cells_arg(c) || !fr->item_mask_sorted)
-        return rl_fail(RL_ERR_ARG, "rl_plus_cell_features: bad argument");
-    if (H != CH) return rl_fail(RL_ERR_ARG, "rl_plus_cell_features: built for hidden_dim 16");
-    if (pna && (!out_sq || !out_min || !out_max || !arg_min || !arg_max || !degree))
-        return rl_fail(RL_ERR_ARG, "rl_plus_cell_features: PNA outputs missing");
-    if (s->num_slots <= 0) return RL_OK;
-    dim3 grid((g->rank_words + PCELL_WARPS - 1) / PCELL_WARPS, s->num_slots);
-    cudaStream_t st = (cudaStream_t)stream;
-#define LAUNCH_PC(CT, P) k_plus_cells<CT, P><<<grid, PCELL_WARPS * 32, 0, st>>>(*g, *r, *s, *fr, *c, emb, out_sum, out_sq, out_min, out_max, arg_min, arg_max, degree)
-    if (fr->count_bits == 32) { if (pna) LAUNCH_PC(uint32_t, true); else LAUNCH_PC(uint32_t, false); }
-    else { if (pna) LAUNCH_PC(unsigned long long, true); else LAUNCH_PC(unsigned long long, false); }
-#undef LAUNCH_PC
-    CHECK_LAUNCH("k_plus_cells");
-    return RL_OK;
-}
-
-int rl_plus_cell_backward(const rl_graph *g, const rl_rules *r, const rl_slots *s, const rl_frontier *fr,
-                          const rl_cells *c, int32_t H, const float *dF, float *grad_emb, void *stream)
-{
-    if (!g || !r || !s || !dF || !grad_emb || bad_frontier(fr) || bad_cells_arg(c) || !fr->item_mask)
-        return rl_fail(RL_ERR_ARG, "rl_plus_cell_backward: bad argument");
-    if (H != CH) return rl_fail(RL_ERR_ARG, "rl_plus_cell_backward: built for hidden_dim 16");
-    if (s->num_slots <= 0) return RL_OK;
-    dim3 grid(PCB_BLOCKS, s->num_slots);
-    cudaStream_t st = (cudaStream_t)stream;
-    if (fr->count_bits == 32) k_plus_cells_bwd<uint32_t><<<grid, WARPS_PER_BLOCK * 32, 0, st>>>(*g, *r, *s, *fr, *c, dF, grad_emb);
-    else k_plus_cells_bwd<unsigned long long><<<grid, WARPS_PER_BLOCK * 32, 0, st>>>(*g, *r, *s, *fr, *c, dF, grad_emb);
-    CHECK_LAUNCH("k_plus_cells_bwd");
-    return RL_OK;
-}
-
-static int no_item_arg(const rl_frontier *fr)
-{
-    return !fr || !fr->arena || !fr->items || !fr->item_off || !fr->item_cnt || !fr->item_mask ||
-           (fr->count_bits != 32 && fr->count_bits != 64);
 }
 
 /* F must hold cap*16 floats; it is cleared here */

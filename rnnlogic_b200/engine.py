@@ -151,10 +151,11 @@ class Grounder:
             raise ValueError("empty batch")
         return np.array(sh, dtype=np.int64), np.array(qo, dtype=np.int64), np.array(gp, dtype=np.int32), pos
 
-    def make_slots(self, heads: Sequence[int], sizes: Sequence[int], all_h, all_t=None, etr=None) -> Slots:
+    def make_slots(self, heads: Sequence[int], sizes: Sequence[int], all_h, all_t=None, etr=None,
+                   coo_only: bool = False) -> Slots:
         """heads[i] / sizes[i]: head relation and number of queries of the i-th single-relation
         group; queries are consecutive in all_h / all_t / etr (int64 CUDA tensors).  Groups larger
-        than 32 are split into several slots."""
+        than 32 are split into several slots.  coo_only: the frontier is for the cell kernels (see make_slots_host)."""
         for name, t in (("all_h", all_h), ("all_t", all_t), ("edges_to_remove", etr)):
             if t is not None:
                 _lib.require_cuda(t, name)
@@ -163,8 +164,10 @@ class Grounder:
             if t is not None and int(t.numel()) != pos:
                 raise ValueError("%s has %d entries for %d queries" % (name, int(t.numel()), pos))
         host = HostStep(self.cr, sh, qo, group_ptr=gp if len(sh) != len(sizes) else None, group_sizes=list(sizes))
-        return Slots(self.dg, host, all_h.contiguous(), None if all_t is None else all_t.contiguous(),
-                     None if etr is None else etr.contiguous())
+        sl = Slots(self.dg, host, all_h.contiguous(), None if all_t is None else all_t.contiguous(),
+                   None if etr is None else etr.contiguous())
+        sl.coo_only = bool(coo_only)
+        return sl
 
     def pack_host(self, batches, with_etr: bool, etr_lists=None) -> HostStep:
         """The CUDA-free half of make_slots_host (thread-safe: a loader thread may run it ahead of the step)."""
@@ -246,6 +249,7 @@ class Grounder:
         sl.cell_counters = sl.state[lay["o_ctr"]:lay["o_ctr"] + 8]
         sl.slot_ncell = scratch[lay["o_ncell"]:lay["o_ncell"] + sl.S]
         sl.flags = sl.state[lay["o_ctr"]:]                 # cell counters[8] | count overflow | non-zero rows per depth[8]: one D2H read
+        sl.nzmask = sl.state[lay["o_nz"]:lay["o_ctr"]].view(sl.S, -1)     # candidate word of every (slot, entity)
         base, sb = sl.state.data_ptr(), scratch.data_ptr()
         coo_only = bool(getattr(sl, "coo_only", False))                  # cell paths: no entity-grouped copy of the items
         sl.frontier = _lib.RlFrontier(bits, sl.arena.data_ptr(), base, base + 4 * lay["o_cnt"],
@@ -298,29 +302,39 @@ class Grounder:
     # ---- candidate cells (rl_cells) ------------------------------------------------------------
     cells_per_slot_hint = 24576       # first guess of the per-cell capacity; grows on demand (see ensure_cell_cap)
 
-    def cell_arrays(self, sl: Slots, floats_per_cell: int):
-        """Grow-only per-cell workspace: int32 keys [cap] + ``floats_per_cell`` fp32 planes [cap] each."""
-        want = (max(self.cell_cap, self.cells_per_slot_hint * sl.S) + 63) // 64 * 64       # planes stay 16-byte aligned
-        n = want * (1 + floats_per_cell)
+    def cell_capacity(self, sl: Slots) -> int:
+        """Cells the per-cell arrays of a call are sized for: the largest count seen so far or the per-slot hint."""
+        return (max(self.cell_cap, self.cells_per_slot_hint * sl.S) + 63) // 64 * 64       # planes stay 16-byte aligned
+
+    def cell_arrays(self, sl: Slots, planes: int):
+        """Grow-only per-cell workspace of ``planes`` 32-bit planes [cap] each -> (cap, flat fp32 tensor)."""
+        want = self.cell_capacity(sl)
+        n = want * planes
         if self._ws_cells is None or self._ws_cells.numel() < n or self._ws_cells_cap < want:
             self._ws_cells = None
             self._ws_cells = torch.empty(n, dtype=torch.float32, device=self.device)
             self._ws_cells_cap = want
             self.generation += 1
-        cap = self._ws_cells_cap
-        planes = [self._ws_cells[(1 + i) * cap:(2 + i) * cap] for i in range(floats_per_cell)]
-        return cap, self._ws_cells[:cap].view(torch.int32), planes
+        return self._ws_cells_cap, self._ws_cells
 
-    def build_cells(self, sl: Slots, floats_per_cell: int):
-        """rl_cells_build for an expanded frontier -> (RlCells, fp32 planes [cap] each)."""
-        cap, keys, planes = self.cell_arrays(sl, 1 + floats_per_cell)      # plane 0: the cells' entities
+    def build_cells(self, sl: Slots, floats_per_cell: int, cap: Optional[int] = None):
+        """rl_cells_build for an expanded frontier -> (RlCells, fp32 planes [floats_per_cell][cap]).
+        cap=None: the arrays live in the grounder's grow-only workspace, which the next call reuses (fused steps
+        consume them within the call).  Else fresh arrays for ``cap`` cells that belong to ``sl`` alone."""
+        if cap is None:
+            cap, ws = self.cell_arrays(sl, 2 + floats_per_cell)
+        else:
+            cap = (max(1, int(cap)) + 63) // 64 * 64
+            ws = torch.empty(cap * (2 + floats_per_cell), dtype=torch.float32, device=self.device)
+        sl.cell_ws = ws                                                   # keeps the arrays alive as long as the call
+        keys, ents = ws[:cap].view(torch.int32), ws[cap:2 * cap]          # plane 1: the cells' entities
         t = sl.cells_tables
-        sl.cells = _lib.RlCells(cap, t["counters"], t["nzmask"], t["cand_off"], keys.data_ptr(), planes[0].data_ptr(),
+        sl.cells = _lib.RlCells(cap, t["counters"], t["nzmask"], t["cand_off"], keys.data_ptr(), ents.data_ptr(),
                                 t["slot_ncell"], t["qmax"], t["qsum"])
         sl.cell_cap = cap
         _lib.check(_lib.lib().rl_cells_build(self.dg.ref(), self.dr.ref(), sl.ref(), sl.fref(), C.byref(sl.cells), _stream()),
                    "rl_cells_build")
-        return sl.cells, planes[1:]
+        return sl.cells, ws[2 * cap:(2 + floats_per_cell) * cap].view(floats_per_cell, cap)
 
     def note_cell_count(self, n_cells: int):
         """Remember the largest cell count seen so that later calls size their arrays for it (x1.25)."""

@@ -90,14 +90,6 @@ class ScoreKernels:
             G.data_ptr() if G is not None else None, _stream()), "rl_softmax_ce")
         return out[0], out[1], G
 
-    # ---- kernel (2c) -------------------------------------------------------------------------
-    def predictor_backward(self, sl: Slots, G, slot_scale: Optional[torch.Tensor], grad_w: torch.Tensor,
-                           grad_bias: Optional[torch.Tensor]):
-        _lib.check(_lib.lib().rl_predictor_backward(
-            self.dg.ref(), self.dr.ref(), sl.ref(), sl.fref(), G.data_ptr(),
-            slot_scale.data_ptr() if slot_scale is not None else None, grad_w.data_ptr(),
-            grad_bias.data_ptr() if grad_bias is not None else None, _stream()), "rl_predictor_backward")
-
     # ---- kernel (3) --------------------------------------------------------------------------
     def filtered_rank(self, sl: Slots, Z, nzmask, which: str, use_mask: bool) -> torch.Tensor:
         """int64[S*32, 2] (L,H) per lane (0,0 on padding lanes); which = 'hr2oo' | 'hr2ooo'."""

@@ -55,36 +55,13 @@ class _RuleModel(nn.Module):
             self._drivers[key] = ScoreKernels(Grounder(self.graph, self.compiled, device, self.force_dense))
         return self._drivers[key]
 
-    def _ground(self, all_h, all_r, edges_to_remove):
+    def _ground(self, all_h, all_r, edges_to_remove, coo_only=False):
         query_r = all_r[0].item()
         assert (all_r != query_r).sum() == 0
         sk = self._driver(all_r.device)
-        sl = sk.gr.make_slots([query_r], [all_h.size(0)], all_h, None, edges_to_remove)
+        sl = sk.gr.make_slots([query_r], [all_h.size(0)], all_h, None, edges_to_remove, coo_only=coo_only)
         sk.gr.ground(sl)
         return query_r, sk, sl
-
-
-class _PredictorScoreFn(torch.autograd.Function):
-    """score = sum_rule w_rule * count_rule (+ bias): kernels (2a) forward / (2c) backward."""
-
-    @staticmethod
-    def forward(ctx, rule_weights, bias, sk, sl, fill_neg_inf):
-        Z, nzmask = sk.predictor_scores(sl, rule_weights.detach().contiguous(),
-                                        None if bias is None else bias.detach().contiguous(), fill_neg_inf)
-        score, nz = sk.to_dense(sl, Z, nzmask)
-        ctx.sk, ctx.sl, ctx.has_bias = sk, sl, bias is not None
-        ctx.nrules = rule_weights.shape[0]
-        ctx.mark_non_differentiable(nz)
-        return score, nz
-
-    @staticmethod
-    def backward(ctx, gscore, _gnz):
-        sk, sl = ctx.sk, ctx.sl
-        G = sk.from_dense(sl, gscore.contiguous())
-        grad_w = torch.zeros(ctx.nrules, dtype=torch.float32, device=gscore.device)
-        grad_b = torch.zeros(sk.N, dtype=torch.float32, device=gscore.device) if ctx.has_bias else None
-        sk.predictor_backward(sl, G, None, grad_w, grad_b)
-        return grad_w, grad_b, None, None, None
 
 
 class Predictor(_RuleModel):
@@ -107,11 +84,10 @@ class Predictor(_RuleModel):
         return self.bias.device if self.entity_feature == "bias" else torch.device("cpu")
 
     def forward(self, all_h, all_r, edges_to_remove):
-        query_r, sk, sl = self._ground(all_h, all_r, edges_to_remove)
+        query_r, sk, sl = self._ground(all_h, all_r, edges_to_remove, coo_only=True)
         use_bias = self.entity_feature == "bias"
-        score, nz = _PredictorScoreFn.apply(self.rule_weights, self.bias if use_bias else None, sk, sl,
-                                            not use_bias)
-        if not bool(nz.any().item()):                                   # predictors.py:67-71
+        score, nz, n_cells = cellpath.predictor_api_scores(self, sk, sl)
+        if n_cells == 0:                                                # predictors.py:67-71
             if use_bias:
                 return score, torch.ones_like(nz)
             return torch.full_like(score, float("inf")), torch.zeros_like(nz)
@@ -131,17 +107,14 @@ class Predictor(_RuleModel):
         if len(ids) == 0:
             return None, None
         sk = self._driver(device)
-        sl = sk.gr.make_slots([query_r], [all_h.size(0)], all_h, all_t.to(device), edges_to_remove)
+        sl = sk.gr.make_slots([query_r], [all_h.size(0)], all_h, all_t.to(device), edges_to_remove, coo_only=True)
         sk.gr.ground(sl)
+        sk.gr.build_cells(sl, 0, cap=1)               # for the candidate words sl.nzmask; the cell numbering is not read
+        nzmask = sl.nzmask
         cr = self.compiled
-        R = self.num_relations
         n_terms = max(1, int(cr.head_terms[query_r]))
         stats = torch.zeros(2, sl.S, n_terms, LANES, dtype=torch.float64, device=device)
-        nzmask = torch.empty(sl.S, sk.N, dtype=torch.int32, device=device)
-        cand_cnt = torch.empty(sl.S * sk.N, dtype=torch.int32, device=device)
         L = _lib.lib()
-        _lib.check(L.rl_plus_mask(sk.dg.ref(), sk.dr.ref(), sl.ref(), sl.fref(), nzmask.data_ptr(), cand_cnt.data_ptr(),
-                                  _stream()), "rl_plus_mask")
         _lib.check(L.rl_rule_stats(sk.dg.ref(), sk.dr.ref(), sl.ref(), sl.fref(), n_terms, stats[0].data_ptr(),
                                    stats[1].data_ptr(), _stream()), "rl_rule_stats")
         B = all_h.size(0)
@@ -482,48 +455,6 @@ class _PlusAggregateFn(torch.autograd.Function):
         return g, None
 
 
-class _SumTailFn(torch.autograd.Function):
-    """Fused dense tail for the `sum` aggregator (kernels rl_sum_tail_forward / _backward):
-    z = MLP([relu(LN(Linear(F))), relation_emb[head]]) per candidate."""
-
-    @staticmethod
-    def forward(ctx, F_, cand_head, W0, b0, gamma, beta, W1, b1, W2, b2, rel_w):
-        C_, H = F_.shape
-        J = W1.shape[0]
-        ts = [t.detach().contiguous().float() for t in (F_, W0, b0, gamma, beta, W1, b1, W2, b2, rel_w)]
-        z = torch.empty(C_, dtype=torch.float32, device=F_.device)
-        _lib.check(_lib.lib().rl_sum_tail_forward(C_, H, J, ts[0].data_ptr(), cand_head.data_ptr(),
-                                                  *[t.data_ptr() for t in ts[1:]], z.data_ptr(), _stream()),
-                   "rl_sum_tail_forward")
-        ctx.save_for_backward(cand_head, *ts)
-        return z
-
-    @staticmethod
-    def backward(ctx, dz):
-        cand_head, F_, W0, b0, gamma, beta, W1, b1, W2, b2, rel_w = ctx.saved_tensors
-        C_, H = F_.shape
-        J = W1.shape[0]
-        dev = F_.device
-        dz = dz.contiguous().float()
-        dF = torch.empty_like(F_)
-        delta1 = torch.empty(C_, J, dtype=torch.float32, device=dev)
-        U = torch.empty(C_, 2 * H, dtype=torch.float32, device=dev)
-        dY = torch.empty_like(F_)
-        dRel = torch.empty_like(F_)
-        g_small = torch.zeros(3 * H + 2 * J + 1, dtype=torch.float32, device=dev)
-        _lib.check(_lib.lib().rl_sum_tail_backward(
-            C_, H, J, F_.data_ptr(), cand_head.data_ptr(), W0.data_ptr(), b0.data_ptr(), gamma.data_ptr(),
-            beta.data_ptr(), W1.data_ptr(), b1.data_ptr(), W2.data_ptr(), b2.data_ptr(), rel_w.data_ptr(),
-            dz.data_ptr(), dF.data_ptr(), delta1.data_ptr(), U.data_ptr(), dY.data_ptr(), dRel.data_ptr(),
-            g_small.data_ptr(), _stream()), "rl_sum_tail_backward")
-        dW1 = delta1.t() @ U                                   # the three outer-product gradients: one GEMM each
-        dW0 = dY.t() @ F_
-        drel = torch.zeros_like(rel_w).index_add_(0, cand_head.long(), dRel)
-        db0, dgamma, dbeta = g_small[:H], g_small[H:2 * H], g_small[2 * H:3 * H]
-        db1, dW2, db2 = g_small[3 * H:3 * H + J], g_small[3 * H + J:3 * H + 2 * J], g_small[3 * H + 2 * J:]
-        return dF, None, dW0, db0, dgamma, dbeta, dW1, db1, dW2.view(1, J), db2, drel
-
-
 class _PlusScatterFn(torch.autograd.Function):
     """candidate scores (+ bias, + entity-feature logits) -> entity-major logits Z[S][N][32]."""
 
@@ -621,7 +552,6 @@ class _LstmEncodeFn(torch.autograd.Function):
 
 
 class PredictorPlus(_RuleModel):
-    fused_tail = True         # `sum` aggregator: run the dense tail in the fused CUDA kernels (rl_tail.cu)
     fused_rnn = True          # `lstm` rule encoder with hidden_dim 16 / 32: rl_rnn.cu instead of cuDNN
 
     def __init__(self, graph, type='emb', num_layers=3, hidden_dim=16, entity_feature='bias', aggregator='sum',
@@ -709,7 +639,7 @@ class PredictorPlus(_RuleModel):
         idx = idx.unsqueeze(-1).unsqueeze(-1).expand(-1, -1, self.hidden_dim)
         return torch.gather(output, 1, idx).squeeze(1)
 
-    # ---- shared by the API forward and the fused trainer paths ---------------------------------
+    # ---- the shapes the cell kernels do not take (cellpath.plus_cells_supported): forward and fused steps ----
     def _logits(self, sk, sl):
         """Z[S][N][32] (autograd-connected to every parameter), nzmask[S][N]."""
         device = sk.device
@@ -732,36 +662,29 @@ class PredictorPlus(_RuleModel):
             stats = _PlusAggregateFn.apply(emb, pc)
             qhead = torch.from_numpy(np.repeat(sl.heads, sl.nq)).to(device)
             cand_head = qhead[pc.cand_query]
-            sm = self.score_model
-            fused_tail = (self.fused_tail and self.aggregator == 'sum' and H in (16, 32) and len(sm.layers) == 2
-                          and sm.layers[1].out_features == 1 and sm.layers[0].out_features <= 256
-                          and sm.batch_norms is None and not sm.short_cut and sm.dropout is None)
-            if fused_tail:
-                r2e = self.rule_to_entity
-                lin0 = r2e.add_model.layers[0]
-                zc = _SumTailFn.apply(stats[0], cand_head.to(torch.int32), lin0.weight, lin0.bias,
-                                      r2e.layer_norm.weight, r2e.layer_norm.bias, sm.layers[0].weight,
-                                      sm.layers[0].bias, sm.layers[1].weight, sm.layers[1].bias,
-                                      self.relation_emb.weight)
+            if self.aggregator == 'sum':
+                out = self.rule_to_entity.post(stats[0])
             else:
-                if self.aggregator == 'sum':
-                    out = self.rule_to_entity.post(stats[0])
-                else:
-                    out = self.rule_to_entity.post(stats[0], stats[1], stats[2], stats[3], pc.degree, pc.cand_query,
-                                                   int(sl.q_off[-1]))
-                rel = self.relation_emb(cand_head)
-                zc = self.score_model(torch.cat([out, rel], dim=-1)).squeeze(-1)
+                out = self.rule_to_entity.post(stats[0], stats[1], stats[2], stats[3], pc.degree, pc.cand_query,
+                                               int(sl.q_off[-1]))
+            rel = self.relation_emb(cand_head)
+            zc = self.score_model(torch.cat([out, rel], dim=-1)).squeeze(-1)
         bias = self.bias if ef == 'bias' else None
         extra = self.RotatE.slot_scores(sk, sl) if ef == 'RotatE' else None
         Z = _PlusScatterFn.apply(zc, bias, extra, pc, ef not in ('bias', 'RotatE'))
         return Z, pc
 
     def forward(self, all_h, all_r, edges_to_remove):
-        query_r, sk, sl = self._ground(all_h, all_r, edges_to_remove)
-        Z, pc = self._logits(sk, sl)
-        score, nz = _ToDenseFn.apply(Z, pc.nzmask, sk, sl)
+        if cellpath.plus_cells_supported(self):
+            query_r, sk, sl = self._ground(all_h, all_r, edges_to_remove, coo_only=True)
+            score, nz, n_cells = cellpath.plus_api_scores(self, sk, sl)
+        else:
+            query_r, sk, sl = self._ground(all_h, all_r, edges_to_remove)
+            Z, pc = self._logits(sk, sl)
+            score, nz = _ToDenseFn.apply(Z, pc.nzmask, sk, sl)
+            n_cells = pc.C
         dense_feature = self.entity_feature in ('bias', 'RotatE')
-        if pc.C == 0 and not dense_feature:                              # predictors.py:236-237
+        if n_cells == 0 and not dense_feature:                           # predictors.py:236-237
             return torch.full_like(score, float("inf")), torch.zeros_like(nz)
         if dense_feature:
             return score, torch.ones_like(nz)

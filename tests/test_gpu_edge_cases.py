@@ -152,39 +152,3 @@ def test_device_lookup_of_the_removed_query_edge(world):
     sk.gr.ground(sl2)
     Zb, _ = sk.predictor_scores(sl2, m.rule_weights.detach(), m.bias.detach(), False)
     assert torch.equal(Za, Zb)
-
-
-@pytest.mark.parametrize("ef", ["bias", "none"])
-def test_fused_ce_backward_equals_separate_calls(world, ef):
-    """rl_predictor_ce_backward (partials from the scores kernel, gradient + bias sweep fused) against
-    rl_softmax_ce + rl_predictor_backward on the same frontier."""
-    from rnnlogic_b200.predictors import Predictor, _group_ptr
-    kg, okg, rules, tri = world
-    torch.manual_seed(5)
-    m = Predictor(kg, ef)
-    m.set_rules(rules)
-    with torch.no_grad():
-        m.rule_weights.copy_(torch.randn(len(rules)) * 0.3)
-        if ef == "bias":
-            m.bias.copy_(torch.randn(kg.entity_size) * 0.3)
-    m = m.cuda()
-    sk = m._driver(torch.device(DEV))
-    batches = [tri[tri[:, 1] == q][:40].astype(np.int64) for q in range(5)]      # 40 > 32: groups of two slots
-    sl = sk.gr.make_slots_host(batches, with_etr=True)
-    sk.gr.ground(sl)
-    gptr, ng = _group_ptr(sl, sk.device)
-    w = m.rule_weights.detach()
-    b = m.bias.detach() if ef == "bias" else None
-    scale = sk.slot_scale(sl.S, 0.25)
-    gw1, gb1 = torch.zeros_like(w), (torch.zeros_like(b) if b is not None else None)
-    loss1, tsum1, _ = sk.predictor_train_tail(sl, w, b, 0.2, gptr, ng, scale, gw1, gb1)
-    loss1, tsum1 = loss1.clone(), tsum1.clone()
-    Z, nz = sk.predictor_scores(sl, w, b, b is None)
-    loss2, tsum2, G = sk.softmax_ce(sl, Z, nz, 0.2, b is None, gptr, ng, want_grad=True)
-    gw2, gb2 = torch.zeros_like(w), (torch.zeros_like(b) if b is not None else None)
-    sk.predictor_backward(sl, G, scale, gw2, gb2)
-    np.testing.assert_allclose(loss1.cpu().numpy(), loss2.cpu().numpy(), rtol=1e-6, atol=1e-7)
-    np.testing.assert_array_equal(tsum1.cpu().numpy(), tsum2.cpu().numpy())
-    np.testing.assert_allclose(gw1.cpu().numpy(), gw2.cpu().numpy(), rtol=1e-5, atol=1e-7)
-    if b is not None:
-        np.testing.assert_allclose(gb1.cpu().numpy(), gb2.cpu().numpy(), rtol=1e-5, atol=1e-7)

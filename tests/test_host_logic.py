@@ -23,7 +23,7 @@ def test_cabi_library_exports_every_declared_symbol():
     for name in sorted(declared):
         assert hasattr(L, name), "missing export " + name
     assert declared == set(_lib.exported_symbols()), declared ^ set(_lib.exported_symbols())
-    assert _lib.lib().rl_abi_version() == 4
+    assert _lib.lib().rl_abi_version() == 5
     if not torch.cuda.is_available():           # no compute without a GPU -- and no silent fallback
         assert _lib.lib().rl_device_count() < 0
         assert b"no CPU fallback" in _lib.lib().rl_last_error()
