@@ -6,6 +6,7 @@
 // so every frontier / logit access is one coalesced 128-byte line.  This is HBM/L2-bound
 // integer work: no tensor cores, the levers are coalescing, loads in flight and grid sizing.
 #include "rl_device.cuh"
+#include <limits.h>
 #include <stdlib.h>
 
 static thread_local char g_err[512] = "";
@@ -73,7 +74,8 @@ __global__ void k_prepare_slots(rl_graph g, int S, const int32_t *__restrict__ s
 //              source is a tail of the parent relation, already resolved to parent rows), coalesced
 //              fetch, one parent-bitmap word per entry, then the live parent rows are pulled (128 B
 //              each, lane = query, 8 loads in flight) and reduced per destination row.
-//              Depth 1: each lane looks the row up in the sorted forward list of its own query entity.
+//              Depth 1: each lane finds the tile's rows in the sorted forward list of its own query entity
+//              (one binary search per tile and lane, then a merge).
 //              Rows outside the bitmap are never written or read.  The query's own edge is cut with
 //              an exact integer fix-up.
 // ------------------------------------------------------------------------------------------
@@ -235,29 +237,60 @@ __device__ __forceinline__ uint32_t numeric_rows(const rl_graph &g, const rl_rul
 
     constexpr bool SEARCH = ROOT && PRUNE;                    // dense mode (every row of a node) keeps the streaming in-edge scan
     if (SEARCH) {
-        // Depth 1: the count of row d for query b is the multiplicity of the edge (h_b -> d).  Each lane searches d in the
-        // SORTED forward list of its own h under this relation (forward DCSR) instead of the warp scanning every in-edge
-        // of d for the 32 sources that matter: log(out-degree of h) steps per row, independent of the row's in-degree.
-        int fs = 0, fe = 0;
-        if (h >= 0) {
-            const int sr = srank_row(g, rho, h);
+        // Depth 1: the count of row d for query b is the multiplicity of the edge (h_b -> d), found in the SORTED
+        // forward list of h_b under this relation (forward DCSR).  The tile's rows ascend with the lane (the active
+        // lanes are a prefix), so each lane finds the part of its list inside [first row, last row] of the tile with
+        // ONE binary search and matches those few entries to the tile's rows by a search over the lanes -- instead of
+        // one search per (row, lane): most rows are non-zero for one or two queries only.
+        auto own_edges = [&](int &fs, int &fe) {             // h's forward list under this relation
+            fs = fe = 0;
+            const int sr = h >= 0 ? srank_row(g, rho, h) : -1;
             if (sr >= 0) {
                 const int fb = g.fsrc_ptr[rho] + sr;
                 fs = g.frow_start[fb];
                 fe = g.frow_start[fb + 1];
             }
+        };
+        int lo, fe;
+        own_edges(lo, fe);
+        const uint32_t act = __ballot_sync(FULL, active);
+        const int key = active ? myrow : INT_MAX;
+        const int r_lo = __shfl_sync(FULL, myrow, 0), r_hi = __shfl_sync(FULL, myrow, __popc(act) - 1);
+        for (int hi = fe; lo < hi;) {
+            const int mid = (lo + hi) >> 1;
+            if (__ldg(g.fedge_dstrow + mid) < r_lo) lo = mid + 1; else hi = mid;
         }
-        for (uint32_t act = __ballot_sync(FULL, active); act; act &= act - 1) {
-            const int j = __ffs(act) - 1;
-            const int rj = __shfl_sync(FULL, myrow, j);
-            int lo = fs, hi = fe;
-            while (lo < hi) {
-                const int mid = (lo + hi) >> 1;
-                if (__ldg(g.fedge_dstrow + mid) < rj) lo = mid + 1; else hi = mid;
+        uint32_t hit = 0;                                    // bit j: the edge (h -> row of lane j) exists
+        bool multi = false;                                  // ... more than once (parallel edges)
+        int d = lo < fe ? __ldg(g.fedge_dstrow + lo) : INT_MAX;
+        while (__any_sync(FULL, d <= r_hi)) {
+            int j = 0;                                       // #lanes whose row is < d
+#pragma unroll
+            for (int step = 16; step > 0; step >>= 1)
+                if (__shfl_sync(FULL, key, j + step - 1) < d) j += step;
+            const bool match = __shfl_sync(FULL, key, j & 31) == d && j < 32 && d <= r_hi;
+            if (match) {
+                multi |= (hit >> j) & 1u;
+                hit |= 1u << j;
             }
-            int cnt = 0;
-            while (lo + cnt < fe && __ldg(g.fedge_dstrow + lo + cnt) == rj) ++cnt;
-            acc = (unsigned long long)cnt;
+            if (d <= r_hi) d = ++lo < fe ? __ldg(g.fedge_dstrow + lo) : INT_MAX;
+        }
+        for (uint32_t todo = act; todo; todo &= todo - 1) {
+            const int j = __ffs(todo) - 1;
+            const int rj = __shfl_sync(FULL, myrow, j);
+            acc = (hit >> j) & 1u;
+            if (multi && acc) {                              // a repeated triple (KnowledgeGraph rejects them): count it
+                int a, b;
+                own_edges(a, b);
+                const int end = b;
+                while (a < b) {
+                    const int mid = (a + b) >> 1;
+                    if (__ldg(g.fedge_dstrow + mid) < rj) a = mid + 1; else b = mid;
+                }
+                int cnt = 0;
+                while (a + cnt < end && __ldg(g.fedge_dstrow + a + cnt) == rj) ++cnt;
+                acc = (unsigned long long)cnt;
+            }
             flush(j);
         }
     } else {
